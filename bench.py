@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # the B200 path (this repo)
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port on host cores
   python bench.py --scaling weak --gpus N ...              # C5: 8M dofs per GPU, lake fill-drain pulse
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of reference source/solvers.py:179-229 (Newton solve for N with F+J
 assembly and the Krylov/AMG linear solves, then the q / melt_n / b nodal updates) on the
@@ -55,6 +56,10 @@ def parse():
     ap.add_argument("--e2e-variant", default="both", choices=["both", "h2d", "d2h", "none"],
                     help="diagnostic: which host copies the end-to-end leg performs")
     ap.add_argument("--no-kernels", action="store_true", help="skip the per-kernel roofline timings")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one left to the caller as DIR/<name>.npy (float64): "
+                         "the fields N, b, qx, qy, melt_n (on meshes above 2^20 vertices the same seeded sample of 2^20 "
+                         "vertices in every run) and the Newton iterations of the timed steps")
     return ap.parse_args()
 
 
@@ -259,6 +264,30 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------ B200 arm
+DUMP_SAMPLE = 1 << 20          # vertices per dumped field: five float64 fields stay at 40 MB
+
+
+def dump_outputs(m, its, out_dir, dist, rank):
+    """--dump-outputs: the state the timed steps hand back to their caller (N, b, q, melt_n) and their Newton
+    iteration counts, so that two builds run with the same arguments can be compared output for output."""
+    import torch
+    n = m.n_vert
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    q = m.get_flux()
+    out = {k: m.get_field(k)[idx] for k in ("N", "b", "melt_n")}
+    out["qx"], out["qy"] = q[idx, 0], q[idx, 1]
+    if dist is not None:           # each rank returns its owned vertices and zeros elsewhere
+        for k, v in out.items():
+            t = torch.from_numpy(np.ascontiguousarray(v)).cuda()
+            dist.all_reduce(t)
+            out[k] = t.cpu().numpy()
+    out["newton_its"] = np.asarray(its, dtype=np.float64)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, f"{k}.npy"), np.asarray(v, dtype=np.float64))
+
+
 def main():
     args = parse()
     if args.impl == "reference":
@@ -369,6 +398,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     ms = maxr(ms)
     st1 = m.stats()
+    if args.dump_outputs:
+        dump_outputs(m, its, args.dump_outputs, dist, rank)
     value = args.steps / (ms / 1e3)
     launches = st1["kernel_launches"] - st0["kernel_launches"]
 
