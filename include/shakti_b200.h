@@ -266,6 +266,44 @@ int shakti_save_outputs_async(shakti_model* m, double* b_out, double* N_out, dou
 /* Page-locked host memory for those buffers (cudaMallocHost / cudaFreeHost). */
 int shakti_alloc_pinned(int64_t bytes, void** out);
 int shakti_free_pinned(void* p);
+/* ---------------------------------------------------------------- water-budget diagnostics
+ * One record of SHAKTI_D_COUNT doubles describes the state a Newton solve converged on: the new N with the
+ * lagged b, q, melt_n and N_n the residual was built from (NOT the state after the nodal updates).  Integrals
+ * use the assembly's own quadrature; every value is global (summed / reduced over ranks).  With F~ the residual
+ * without Dirichlet replacement or lifting, sum_i F~_i = int R, which splits into the identity
+ *   outflow = input - (1/rho_i - 1/rho_w) melt + closure + storage + imbalance
+ * that holds at every converged step up to rounding (DESIGN.md, "Water-budget diagnostics"). */
+typedef enum shakti_diag {
+  SHAKTI_D_DT = 0,          /* dt of the solve [s]                                          */
+  SHAKTI_D_NEWTON_ITS = 1,  /* Newton iterations                                            */
+  SHAKTI_D_RESIDUAL = 2,    /* ||F||_2 at exit (stats.last_residual)                        */
+  SHAKTI_D_AREA = 3,        /* int 1 [m^2]                                                  */
+  SHAKTI_D_WATER_VOLUME = 4,/* int b [m^3]                                                  */
+  SHAKTI_D_INPUT = 5,       /* int inputs [m^3/s]                                           */
+  SHAKTI_D_MELT = 6,        /* int (m0 + mdiff) [kg/s]                                      */
+  SHAKTI_D_CLOSURE = 7,     /* int A b N|N|^(n-1) [m^3/s]                                   */
+  SHAKTI_D_STORAGE = 8,     /* int storage (N - N_n) / (rho_w g dt) [m^3/s]                 */
+  SHAKTI_D_OUTFLOW = 9,     /* -sum over Dirichlet rows of F~: discharge through the boundary [m^3/s] */
+  SHAKTI_D_IMBALANCE = 10,  /* sum over the other rows of F~: what Newton left [m^3/s]      */
+  SHAKTI_D_N_MEAN = 11,     /* int N / int 1 [Pa]                                           */
+  SHAKTI_D_N_MIN = 12,      /* min over vertices [Pa]                                       */
+  SHAKTI_D_N_MAX = 13,      /* max over vertices [Pa]                                       */
+  SHAKTI_D_B_MAX = 14,      /* max over vertices [m]                                        */
+  SHAKTI_D_COUNT = 15
+} shakti_diag;
+/* One record of the current state, synchronous (a parity hook): recomputes Kbar; columns 0-2 are dt, 0 and
+ * ||F||_2 of the current state (the residual field is re-assembled). */
+int shakti_diagnostics(shakti_model* m, double dt, double out[SHAKTI_D_COUNT]);
+/* capacity > 0: every converged Newton solve (shakti_newton_solve, shakti_step, shakti_run*, shakti_step_host*)
+ * appends one record to a device buffer of `capacity` rows, on the stream, without a host synchronisation.
+ * 0 (the default): off, a step launches nothing extra.  Rows not yet read are discarded.  A solve that finds
+ * the buffer full fails with SHAKTI_ERR_INVALID before it changes any state; shakti_run checks nsteps
+ * against the free rows up front.  Rows recorded after shakti_snapshot are dropped by shakti_rollback. */
+int shakti_record_diagnostics(shakti_model* m, int64_t capacity);
+/* Copy the recorded rows (row-major, SHAKTI_D_COUNT doubles each; max_rows must hold them all) to `rows` and
+ * empty the buffer; *n_rows = rows copied.  rows == NULL: only query the count (the buffer is kept). */
+int shakti_read_diagnostics(shakti_model* m, double* rows, int64_t max_rows, int64_t* n_rows);
+
 /* Diagnostic: GB/s of cudaMemcpyAsync host->device / device->host for `host` (any host pointer) and the host
  * milliseconds each enqueue took (enqueue_ms[0] h2d, [1] d2h): tells page-locked from pageable memory. */
 int shakti_debug_copy_bw(void* host, int64_t bytes, int reps, double* h2d_gbs, double* d2h_gbs, double* enqueue_ms);
@@ -335,7 +373,9 @@ typedef enum shakti_host_array {
   SHAKTI_HM_AB_HALO = 20,   /* halo vertices per block (local ids)                        */
   SHAKTI_HM_AB_INCPTR = 21, /* n_owned+1                                                  */
   SHAKTI_HM_AB_INC = 22,    /* (cell index in block)*4 + local vertex index               */
-  SHAKTI_HM_AB_SRC = 23     /* per padded SELL entry: two 16-bit gather codes (as int32 bits) */
+  SHAKTI_HM_AB_SRC = 23,    /* per padded SELL entry: two 16-bit gather codes (as int32 bits) */
+  SHAKTI_HM_CELL_COUNTED = 24 /* n_cell_local: 1 on exactly one rank per cell (the owner of its vertex with the
+                                 smallest caller id), else 0: the cells whose integrals this rank contributes */
 } shakti_host_array;
 /* Size query (out == NULL) or copy of one of the arrays above. */
 int shakti_host_mesh_array(shakti_host_mesh* hm, int which, int32_t* out, int64_t* n);

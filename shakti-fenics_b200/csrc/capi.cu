@@ -64,6 +64,12 @@ struct shakti_model {
   double snap_hist_ratio = -1.0, snap_hist_dt = 0.0, snap_residual0 = 0.0;
   int64_t snap_steps = 0;
   bool snap_valid = false;
+  // water-budget diagnostics: cells this rank counts, reduction scratch (partials; rank values + one-shot row)
+  // and the record buffer of diag_cap rows, diag_n of them filled (snap_diag_n at the last snapshot)
+  DevBuf<uint8_t> cell_counted;
+  DevBuf<double> diag_partial, diag_vals, diag_rows;
+  int diag_parts = 1;
+  int64_t diag_cap = 0, diag_n = 0, snap_diag_n = 0;
   double N_bdry = 0.0;
   int64_t n_bc = 0;
   bool h0_dirty = true;
@@ -333,9 +339,30 @@ __global__ void fix_bc_dx_kernel(int32_t n, const uint8_t* __restrict__ isbc, co
 // and the final iterate is solved as tightly as before, so the iteration counts and the converged fields
 // are those of the exact iteration (tests: identical Newton counts, fields <= 1e-8 against the CPU LU
 // restatement) at roughly 60 % of the Krylov iterations.
+// One water-budget record of the current state into `row` (device, SHAKTI_D_COUNT doubles), on the stream.
+// Kbar and h0 must be current.
+static void diagnostics_record(shakti_model* m, double dt, int its, double residual, double* row) {
+  ensure_rules(m);
+  const bool multi = comm().active();
+  launch_diagnostics(m->hm.ne, m->c0.p, m->c1.p, m->c2.p, m->cell_counted.p, m->fields(), m->kbar.p, dt, m->dprm,
+                     m->diag_parts, m->diag_partial.p, m->diag_vals.p, multi ? nullptr : row, its, residual, m->stream);
+  if (multi) {
+    comm_allreduce_sum(m->diag_vals.p, kDiagSums, m->stream);
+    comm_allreduce_max(m->diag_vals.p + kDiagSums, kDiagVals - kDiagSums, m->stream);
+    launch_diagnostics_row(m->diag_vals.p, row, dt, its, residual, m->stream);
+  }
+}
+
+static void require_diag_rows(shakti_model* m, int64_t n) {
+  if (m->diag_cap > 0 && n > m->diag_cap - m->diag_n)
+    throw Error(SHAKTI_ERR_INVALID, "diagnostics buffer full (" + std::to_string(m->diag_n) + " of " +
+                                        std::to_string(m->diag_cap) + " rows): read it with shakti_read_diagnostics");
+}
+
 static void newton_solve(shakti_model* m, double dt, int32_t* niter, int32_t* converged) {
   const int32_t no = m->hm.n_owned;
   static const bool trace = getenv("SHAKTI_TRACE_NEWTON") != nullptr;
+  require_diag_rows(m, 1);
   compute_kbar(m);
   assemble(m, dt, 1);
   double r = norm2(m, m->F.p);
@@ -440,6 +467,10 @@ static void newton_solve(shakti_model* m, double dt, int32_t* niter, int32_t* co
   *niter = it;
   *converged = conv ? 1 : 0;
   if (!conv) throw Error(SHAKTI_ERR_NOT_CONVERGED, "Newton solver did not converge");
+  if (m->diag_cap > 0) {   // Kbar and h0 are those of the solve
+    diagnostics_record(m, dt, it, r, m->diag_rows.p + m->diag_n * SHAKTI_D_COUNT);
+    m->diag_n++;
+  }
 }
 
 static void update_q(shakti_model* m) {
@@ -612,6 +643,10 @@ static void create(int64_t nv, int64_t ne, const double* xy, const int32_t* cell
     std::vector<uint32_t>().swap(m->ab.src);
   }
   m->diag_pos.upload(hm.diag_pos);
+  m->cell_counted.upload(std::vector<uint8_t>(hm.cell_counted.begin(), hm.cell_counted.end()));
+  m->diag_parts = diagnostics_parts(hm.ne, m->sm_count);
+  m->diag_partial.alloc((size_t)m->diag_parts * kDiagVals);
+  m->diag_vals.alloc(kDiagVals + SHAKTI_D_COUNT);
   m->win.upload(hm.win);
   m->l2g.upload(hm.l2g);
   const size_t nl = std::max<int32_t>(hm.n_local, 1);
@@ -1078,6 +1113,7 @@ int shakti_run(shakti_model* m, const double* dts, int64_t nsteps, int32_t* nite
   SHAKTI_TRY
   SHAKTI_REQUIRE(m && dts && nsteps >= 0, "bad arguments");
   use_device(m);
+  require_diag_rows(m, nsteps);
   for (int64_t i = 0; i < nsteps; ++i) {
     int32_t it = 0, cv = 0;
     shakti::step(m, dts[i], &it, &cv);
@@ -1091,6 +1127,7 @@ int shakti_run_timed(shakti_model* m, const double* dts, int64_t nsteps, int32_t
   SHAKTI_TRY
   SHAKTI_REQUIRE(m && dts && nsteps >= 0 && ms, "bad arguments");
   use_device(m);
+  require_diag_rows(m, nsteps);
   cudaEvent_t e0, e1;
   SHAKTI_CUDA(cudaEventCreate(&e0));
   SHAKTI_CUDA(cudaEventCreate(&e1));
@@ -1137,6 +1174,7 @@ int shakti_snapshot(shakti_model* m) {
   }
   m->snap_hist_ratio = m->hist_ratio; m->snap_hist_dt = m->hist_dt; m->snap_residual0 = m->residual0;
   m->snap_steps = m->st.steps;
+  m->snap_diag_n = m->diag_n;
   m->snap_valid = true;
   SHAKTI_CATCH
 }
@@ -1153,6 +1191,48 @@ int shakti_rollback(shakti_model* m) {
   // the step counter goes back too, and the AMG hierarchy (numbers of a later state) is renewed at the next solve
   m->st.steps = m->snap_steps;
   m->step_of_refresh = -1000000;
+  m->diag_n = std::min(m->diag_n, m->snap_diag_n);   // records of the undone solves
+  SHAKTI_CATCH
+}
+
+int shakti_diagnostics(shakti_model* m, double dt, double out[SHAKTI_D_COUNT]) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && out && dt > 0, "bad arguments");
+  use_device(m);
+  compute_kbar(m);
+  assemble(m, dt, 0);
+  const double r = norm2(m, m->F.p);
+  double* row = m->diag_vals.p + kDiagVals;
+  diagnostics_record(m, dt, 0, r, row);
+  SHAKTI_CUDA(cudaMemcpyAsync(out, row, sizeof(double) * SHAKTI_D_COUNT, cudaMemcpyDeviceToHost, m->stream));
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
+  SHAKTI_CATCH
+}
+
+int shakti_record_diagnostics(shakti_model* m, int64_t capacity) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && capacity >= 0 && capacity <= ((int64_t)1 << 40), "bad arguments");
+  use_device(m);
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
+  if (capacity > 0) m->diag_rows.alloc((size_t)capacity * SHAKTI_D_COUNT);
+  else m->diag_rows.release();
+  m->diag_cap = capacity;
+  m->diag_n = m->snap_diag_n = 0;
+  SHAKTI_CATCH
+}
+
+int shakti_read_diagnostics(shakti_model* m, double* rows, int64_t max_rows, int64_t* n_rows) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && n_rows, "null argument");
+  *n_rows = m->diag_n;
+  if (!rows) return SHAKTI_OK;
+  SHAKTI_REQUIRE(max_rows >= m->diag_n, "row buffer too small for the recorded diagnostics");
+  use_device(m);
+  if (m->diag_n)
+    SHAKTI_CUDA(cudaMemcpyAsync(rows, m->diag_rows.p, sizeof(double) * SHAKTI_D_COUNT * m->diag_n, cudaMemcpyDeviceToHost,
+                                m->stream));
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
+  m->diag_n = m->snap_diag_n = 0;
   SHAKTI_CATCH
 }
 
@@ -1505,6 +1585,7 @@ int shakti_host_mesh_array(shakti_host_mesh* h, int which, int32_t* out, int64_t
     case SHAKTI_HM_DIAG_POS: v = &m.diag_pos; break;
     case SHAKTI_HM_WIN: v = &m.win; break;
     case SHAKTI_HM_WIN_CELL: v = &m.win_cell; break;
+    case SHAKTI_HM_CELL_COUNTED: v = &m.cell_counted; break;
     case SHAKTI_HM_NBR_RANK:
       for (const auto& nb : m.nbrs) tmp.push_back(nb.rank);
       v = &tmp; break;

@@ -80,6 +80,25 @@ void launch_assemble_blocks(const AssemblyPlanView& plan, FieldPtrs f, const dou
 void launch_apply_bc(int32_t n_owned, const uint8_t* isbc, const double* N, double N_bdry,
                      const int32_t* diag_pos, double* F, double* Jval, int want_J, cudaStream_t s);
 
+// ---- water-budget diagnostics (shakti_diagnostics, shakti_record_diagnostics)
+// Rank-local values before the global reduction: kDiagSums sums (all-reduced by sum), then maxima (by max;
+// the minimum of N is carried as the maximum of -N).
+enum {
+  kDiagArea = 0, kDiagVolume, kDiagInput, kDiagMelt, kDiagClosure, kDiagStorage, kDiagOutflow, kDiagImbalance, kDiagIntN,
+  kDiagSums,
+  kDiagNegNmin = kDiagSums, kDiagNmax, kDiagBmax,
+  kDiagVals
+};
+// blocks of the cell pass (= partials it writes)
+int diagnostics_parts(int32_t ne, int sm_count);
+// counted: 1 for the local cells this rank adds (prep.h HostMesh::cell_counted); partial: nparts x kDiagVals scratch.
+// Writes the rank's values to vals[kDiagVals] and, if row != NULL, the finished record (one rank only).
+void launch_diagnostics(int32_t ne, const int32_t* c0, const int32_t* c1, const int32_t* c2, const uint8_t* counted, FieldPtrs f,
+                        const double* kbar, double dt, DevParams p, int nparts, double* partial, double* vals, double* row,
+                        double its, double residual, cudaStream_t s);
+// record row from globally reduced vals (several ranks)
+void launch_diagnostics_row(const double* vals, double* row, double dt, double its, double residual, cudaStream_t s);
+
 // ---- nodal updates (solvers.py:186-197)
 void launch_update_q(int32_t n_owned, const int32_t* win, const double* x, const double* y,
                      const double* h0, const double* N, const double* b, double* qx, double* qy,

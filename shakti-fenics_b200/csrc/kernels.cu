@@ -1545,4 +1545,168 @@ void launch_deinterleave(int64_t n, const double* ab, double* a, double* b, cuda
   SHAKTI_LAUNCH(deinterleave_kernel, stream_blocks(n), 256, 0, s, n, ab, a, b);
 }
 
+// ------------------------------------------------------------------ water-budget diagnostics
+// One record of the global water budget at the current state (DESIGN.md "Water-budget diagnostics").  Stage 1:
+// every cell this rank counts (cell_counted) adds its unconstrained element residual F_a (element_core, no
+// lifting) to the outflow (Dirichlet vertex, negated) or to the imbalance (other vertex), its source integrals
+// by the assembly's own rules and its vertex extrema; each block reduces its threads in a fixed tree and
+// writes one partial.  Stage 2: one block sums the partials in a fixed order.  No floating-point atomics, so
+// a record is bitwise reproducible for a given grid.
+constexpr int kDiagThreads = 256;
+
+__device__ __forceinline__ void diag_block_reduce(double (&v)[kDiagVals], double* __restrict__ sh, double* __restrict__ out) {
+  // sh: kDiagVals x kDiagThreads; sums for [0, kDiagSums), maxima after
+#pragma unroll
+  for (int k = 0; k < kDiagVals; ++k) sh[k * kDiagThreads + threadIdx.x] = v[k];
+  __syncthreads();
+  for (int w = kDiagThreads / 2; w > 0; w >>= 1) {
+    if ((int)threadIdx.x < w) {
+#pragma unroll
+      for (int k = 0; k < kDiagVals; ++k) {
+        const double a = sh[k * kDiagThreads + threadIdx.x], b = sh[k * kDiagThreads + threadIdx.x + w];
+        sh[k * kDiagThreads + threadIdx.x] = k < kDiagSums ? a + b : fmax(a, b);
+      }
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < kDiagVals) out[threadIdx.x] = sh[threadIdx.x * kDiagThreads];
+}
+
+__global__ void __launch_bounds__(kDiagThreads)
+diagnostics_kernel(int32_t ne, const int32_t* __restrict__ c0, const int32_t* __restrict__ c1, const int32_t* __restrict__ c2,
+                   const uint8_t* __restrict__ counted, FieldPtrs f, const double* __restrict__ kbar, double dt, DevParams p,
+                   double* __restrict__ partial) {
+  __shared__ double sh[kDiagVals * kDiagThreads];
+  double v[kDiagVals];
+#pragma unroll
+  for (int k = 0; k < kDiagVals; ++k) v[k] = k < kDiagSums ? 0.0 : -INFINITY;
+  const int32_t stride = gridDim.x * blockDim.x;
+  for (int32_t e = blockIdx.x * blockDim.x + threadIdx.x; e < ne; e += stride) {
+    if (!counted[e]) continue;
+    const int32_t vv[3] = {c0[e], c1[e], c2[e]};
+    const Geo g = geometry(f.x[vv[0]], f.y[vv[0]], f.x[vv[1]], f.y[vv[1]], f.x[vv[2]], f.y[vv[2]]);
+    double h[3], bb[3], mm[3], qxv[3], qyv[3], Nv[3], Nn[3], st[3], Gv[3], inp[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      Nv[i] = f.N[vv[i]];
+      h[i] = f.h0[vv[i]] - Nv[i] * p.inv_rwg;
+      bb[i] = f.b[vv[i]];
+      mm[i] = f.melt[vv[i]];
+      qxv[i] = f.qx[vv[i]];
+      qyv[i] = f.qy[vv[i]];
+      Nn[i] = f.N_n[vv[i]];
+      st[i] = f.storage[vv[i]];
+      Gv[i] = f.G[vv[i]];
+      inp[i] = f.inputs[vv[i]];
+    }
+    ElemOut o;
+    element_core(g, h, bb, mm, qxv, qyv, Nv, Nn, st, Gv, inp, kbar[e], dt, p, o);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      if (f.isbc[vv[a]]) v[kDiagOutflow] -= o.F[a];
+      else v[kDiagImbalance] += o.F[a];
+    }
+    // melt m0 + mdiff at the vertices, as element_core forms it (constitutive.py:25-26)
+    double ghx = 0, ghy = 0, gbx = 0, gby = 0, gmx = 0, gmy = 0;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      ghx += h[i] * g.gx[i];  ghy += h[i] * g.gy[i];
+      gbx += bb[i] * g.gx[i]; gby += bb[i] * g.gy[i];
+      gmx += mm[i] * g.gx[i]; gmy += mm[i] * g.gy[i];
+    }
+    const double gb2 = gbx * gbx + gby * gby, gmgb = gmx * gbx + gmy * gby, inv1 = 1.0 / (1.0 + gb2);
+    double smelt = 0, sinp = 0, sb = 0, sN = 0, ss = 0, sd = 0, ssd = 0;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      smelt += (Gv[i] - p.rwg * (qxv[i] * ghx + qyv[i] * ghy)) * p.inv_Lh + (gb2 * mm[i] + bb[i] * gmgb) * inv1;
+      sinp += inp[i];
+      sb += bb[i];
+      sN += Nv[i];
+      const double d = Nv[i] - Nn[i];
+      ss += st[i];
+      sd += d;
+      ssd += st[i] * d;
+    }
+    const double m6 = g.detabs * (1.0 / 6.0);   // int phi_a = |detJ| / 6
+    v[kDiagArea] += 0.5 * g.detabs;
+    v[kDiagVolume] += m6 * sb;
+    v[kDiagInput] += m6 * sinp;
+    v[kDiagMelt] += m6 * smelt;
+    v[kDiagIntN] += m6 * sN;
+    // storage: int s (N - N_n) of two P1 functions, times 1/(rho_w g dt)
+    v[kDiagStorage] += p.inv_rwg / dt * g.detabs * (1.0 / 24.0) * (ss * sd + ssd);
+    // closure A b N|N|^(n-1) by the assembly's rule: Radon-7 for n = 3, the __constant__ table otherwise
+    double clos = 0;
+    if (p.n_is_3) {
+      double f0, f1, f2, m00, m01, m02, m11, m12, m22;
+      reaction_radon7<false>(g.detabs, bb, Nv, Nn, st, 0.0, p.A, f0, f1, f2, m00, m01, m02, m11, m12, m22);
+      clos = f0 + f1 + f2;
+    } else {
+      const double e1 = p.n - 1.0;
+      const int nq = c_nrq;
+      for (int k = 0; k < nq; ++k) {
+        const double l0 = c_rq[4 * k], l1 = c_rq[4 * k + 1], l2 = c_rq[4 * k + 2];
+        const double bq = l0 * bb[0] + l1 * bb[1] + l2 * bb[2];
+        const double Nq = l0 * Nv[0] + l1 * Nv[1] + l2 * Nv[2];
+        clos += c_rq[4 * k + 3] * g.detabs * (p.A * bq * Nq * pow(fabs(Nq), e1));
+      }
+    }
+    v[kDiagClosure] += clos;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      v[kDiagNegNmin] = fmax(v[kDiagNegNmin], -Nv[i]);
+      v[kDiagNmax] = fmax(v[kDiagNmax], Nv[i]);
+      v[kDiagBmax] = fmax(v[kDiagBmax], bb[i]);
+    }
+  }
+  diag_block_reduce(v, sh, partial + (size_t)blockIdx.x * kDiagVals);
+}
+
+// global values vals[kDiagVals] -> one record row[SHAKTI_D_COUNT]
+__device__ __forceinline__ void diag_write_row(const double* vals, double* row, double dt, double its, double residual) {
+  row[SHAKTI_D_DT] = dt;
+  row[SHAKTI_D_NEWTON_ITS] = its;
+  row[SHAKTI_D_RESIDUAL] = residual;
+#pragma unroll
+  for (int k = 0; k <= kDiagImbalance; ++k) row[SHAKTI_D_AREA + k] = vals[k];
+  row[SHAKTI_D_N_MEAN] = vals[kDiagIntN] / vals[kDiagArea];
+  row[SHAKTI_D_N_MIN] = -vals[kDiagNegNmin];
+  row[SHAKTI_D_N_MAX] = vals[kDiagNmax];
+  row[SHAKTI_D_B_MAX] = vals[kDiagBmax];
+}
+
+__global__ void __launch_bounds__(kDiagThreads)
+diagnostics_finish_kernel(int nparts, const double* __restrict__ partial, double* __restrict__ vals, double* __restrict__ row,
+                          double dt, double its, double residual) {
+  __shared__ double sh[kDiagVals * kDiagThreads];
+  double v[kDiagVals];
+#pragma unroll
+  for (int k = 0; k < kDiagVals; ++k) v[k] = k < kDiagSums ? 0.0 : -INFINITY;
+  for (int b = threadIdx.x; b < nparts; b += kDiagThreads)
+#pragma unroll
+    for (int k = 0; k < kDiagVals; ++k) v[k] = k < kDiagSums ? v[k] + partial[(size_t)b * kDiagVals + k] : fmax(v[k], partial[(size_t)b * kDiagVals + k]);
+  diag_block_reduce(v, sh, vals);
+  if (row == nullptr) return;
+  __syncthreads();
+  if (threadIdx.x == 0) diag_write_row(vals, row, dt, its, residual);
+}
+
+__global__ void diagnostics_row_kernel(const double* __restrict__ vals, double* __restrict__ row, double dt, double its,
+                                       double residual) {
+  diag_write_row(vals, row, dt, its, residual);
+}
+
+int diagnostics_parts(int32_t ne, int sm_count) { return std::max(1, std::min(div_up(ne, kDiagThreads), 4 * sm_count)); }
+
+void launch_diagnostics(int32_t ne, const int32_t* c0, const int32_t* c1, const int32_t* c2, const uint8_t* counted, FieldPtrs f,
+                        const double* kbar, double dt, DevParams p, int nparts, double* partial, double* vals, double* row,
+                        double its, double residual, cudaStream_t s) {
+  if (ne > 0) SHAKTI_LAUNCH(diagnostics_kernel, nparts, kDiagThreads, 0, s, ne, c0, c1, c2, counted, f, kbar, dt, p, partial);
+  SHAKTI_LAUNCH(diagnostics_finish_kernel, 1, kDiagThreads, 0, s, ne > 0 ? nparts : 0, partial, vals, row, dt, its, residual);
+}
+
+void launch_diagnostics_row(const double* vals, double* row, double dt, double its, double residual, cudaStream_t s) {
+  SHAKTI_LAUNCH(diagnostics_row_kernel, 1, 1, 0, s, vals, row, dt, its, residual);
+}
+
 }  // namespace shakti

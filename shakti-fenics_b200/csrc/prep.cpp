@@ -623,6 +623,15 @@ void build_host_mesh(int64_t nv, int64_t ne, const double* xy, const int32_t* ce
   }
   });
   lap("winning cells");
+  m.cell_counted.assign(m.ne, 1);
+  if (nranks > 1)
+    parallel_for(m.ne, [&](int64_t e0, int64_t e1, int) {
+      for (int64_t e = e0; e < e1; ++e) {
+        const int32_t* c = m.cells.data() + 3 * (size_t)e;
+        const int32_t g = std::min(m.l2g[c[0]], std::min(m.l2g[c[1]], m.l2g[c[2]]));
+        m.cell_counted[e] = owner_of_pos(posof[g]) == rank ? 1 : 0;
+      }
+    });
   // halo maps
   m.nbrs.clear();
   if (nranks > 1) {

@@ -56,6 +56,9 @@ struct HostMesh {
   std::vector<int32_t> diag_pos;  // n_owned: SELL position of the diagonal
   std::vector<int32_t> win;       // 4 x n_owned: v0,v1,v2 (local ids) of the winning cell, local index
   std::vector<int32_t> win_cell;  // n_owned: caller cell id of the winning cell
+  // ne: 1 if this rank counts the cell in global integrals (it owns the cell's vertex with the smallest caller
+  // id), else 0 -- every cell is counted on exactly one rank although local cells overlap between ranks
+  std::vector<int32_t> cell_counted;
   std::vector<Neighbor> nbrs;
 };
 

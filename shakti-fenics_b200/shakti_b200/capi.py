@@ -19,7 +19,11 @@ PC = dict(jacobi=0, amg=1, none=2)
 NEWTON_R0 = dict(dolfinx=0, initial_residual=1)
 HOST_ARRAYS = dict(l2g=0, cells=1, cell_l2g=2, rowptr=3, col=4, slice_ptr=5, sell_col=6, slot=7, diag_pos=8,
                    win=9, win_cell=10, nbr_rank=11, nbr_send_ptr=12, nbr_send_idx=13, nbr_recv=14,
-                   ab_info=15, ab_eptr=16, ab_elems=17, ab_lv=18, ab_hptr=19, ab_halo=20, ab_incptr=21, ab_inc=22, ab_src=23)
+                   ab_info=15, ab_eptr=16, ab_elems=17, ab_lv=18, ab_hptr=19, ab_halo=20, ab_incptr=21, ab_inc=22, ab_src=23,
+                   cell_counted=24)
+# columns of a water-budget record (enum shakti_diag)
+DIAGNOSTICS = ("dt", "newton_its", "residual", "area", "water_volume", "input", "melt", "closure", "storage", "outflow",
+               "imbalance", "N_mean", "N_min", "N_max", "b_max")
 
 ERR_NOT_CONVERGED = -4
 ERR_LINEAR = -5
@@ -474,6 +478,25 @@ class Model:
     def save_outputs_async(self, b, N, qx, qy, owned_only=False):
         """Enqueue snapshots of b, N, qx, qy into the given (pinned) numpy arrays; valid after wait_outputs()."""
         _check(self.lib.shakti_save_outputs_async(self._h, _p(b), _p(N), _p(qx), _p(qy), C.c_int(1 if owned_only else 0)))
+
+    # ---- water-budget diagnostics (columns: DIAGNOSTICS)
+    def diagnostics(self, dt):
+        """One record of the current state -> dict (columns 0-2: dt, 0, ||F|| of the current state)."""
+        out = np.empty(len(DIAGNOSTICS))
+        _check(self.lib.shakti_diagnostics(self._h, C.c_double(dt), _p(out)))
+        return dict(zip(DIAGNOSTICS, out.tolist()))
+
+    def record_diagnostics(self, capacity):
+        """capacity > 0: every converged Newton solve appends one record on the device; 0: off."""
+        _check(self.lib.shakti_record_diagnostics(self._h, C.c_int64(int(capacity))))
+
+    def read_diagnostics(self):
+        """The recorded rows as an (n, len(DIAGNOSTICS)) array; empties the buffer."""
+        n = C.c_int64(0)
+        _check(self.lib.shakti_read_diagnostics(self._h, None, C.c_int64(0), C.byref(n)))
+        rows = np.empty((n.value, len(DIAGNOSTICS)))
+        _check(self.lib.shakti_read_diagnostics(self._h, _p(rows), C.c_int64(n.value), C.byref(n)))
+        return rows[: n.value]
 
     # ---- micro-benchmarks
     KERNELS = dict(spmv=0, assemble=1, kbar=2, nodal=3, dot=4, axpy=5)

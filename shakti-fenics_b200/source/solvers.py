@@ -334,6 +334,28 @@ def solve(md):
                     arr[:min(arr.shape[0], prev.shape[0])] = prev[:arr.shape[0]]
         j = len(range(0, first, md.nt_save))
 
+    # extension (off unless md.diagnostics_on): one water-budget record per time step (capi.DIAGNOSTICS), recorded on
+    # the device and written by rank 0 to <results>/diagnostics.npz (t and one array per column) at every checkpoint
+    # save and at the end; a resumed run keeps the rows of the steps before `first` from the existing file
+    diag = None
+    if getattr(md, "diagnostics_on", False):
+        solver.model.record_diagnostics(max(nt - first, 1))
+        diag_file = os.path.join(md.results_name, "diagnostics.npz")
+        diag = dict(t=np.zeros(0), rows=np.zeros((0, len(capi.DIAGNOSTICS))), read=0)
+        if first > 0 and md.rank == 0 and os.path.exists(diag_file):
+            prev = np.load(diag_file)
+            diag["t"] = prev["t"][:first]
+            diag["rows"] = np.stack([prev[k] for k in capi.DIAGNOSTICS], axis=1)[:first]
+
+    def save_diagnostics():
+        rows = solver.model.read_diagnostics()      # every rank: the records are global and each rank empties its buffer
+        i0 = first + diag["read"]
+        diag["read"] += rows.shape[0]
+        if md.rank == 0:
+            diag["t"] = np.concatenate([diag["t"], md.timesteps[i0:i0 + rows.shape[0]]])
+            diag["rows"] = np.concatenate([diag["rows"], rows])
+            np.savez(diag_file, t=diag["t"], **dict(zip(capi.DIAGNOSTICS, diag["rows"].T)))
+
     for i in range(first, nt):
 
         if md.rank == 0 and (i + 1) % 10 == 0:
@@ -370,6 +392,8 @@ def solve(md):
                     np.save(md.results_name + '/N.npy', N_arr)
                     np.save(md.results_name + '/qx.npy', qx_arr)
                     np.save(md.results_name + '/qy.npy', qy_arr)
+                if diag is not None:
+                    save_diagnostics()
 
             j += 1
 
@@ -386,6 +410,8 @@ def solve(md):
         np.save(md.results_name + '/N.npy', N_arr)
         np.save(md.results_name + '/qx.npy', qx_arr)
         np.save(md.results_name + '/qy.npy', qy_arr)
+    if diag is not None:
+        save_diagnostics()
 
     solver.pull()
     md.final = dict(N=N, N_n=N_n, b=b, q=q, melt_n=melt_n)
