@@ -290,9 +290,8 @@ amg_spgemm_table_kernel(SellView A, const int32_t* __restrict__ Alen, SellView B
 static void build_spgemm_plan(const DevSell& A, const DevSell& B, const DevSell& C, SpgemmPlan& plan, cudaStream_t s) {
   plan.built = true;
   plan.ok = false;
-  static const bool disabled = getenv("SHAKTI_SPGEMM_SEARCH") != nullptr;   // A/B switch: keep the searching kernels
   const size_t smem = (size_t)C.max_width * 128 * sizeof(double);
-  if (disabled || A.n_rows == 0 || C.max_width > 255 || smem > 96 * 1024) return;
+  if (A.n_rows == 0 || C.max_width > 255 || smem > 96 * 1024) return;
   DevBuf<int32_t> width;
   width.alloc_zero(A.n_slices, s);
   SHAKTI_LAUNCH(amg_spgemm_count_kernel, div_up((int64_t)A.n_slices * 32, 128), 128, 0, s, view(A), A.rowlen.p, B.rowlen.p, B.n_rows,

@@ -47,7 +47,6 @@ struct shakti_model {
   // vertex fields (n_local)
   DevBuf<double> z_b, z_s, h0, G, inputs, storage, b, b2, N, N_n, qx, qy, melt, melt2, F, dx, rhs, dinv;
   DevBuf<double> kbar;
-  DevBuf<double> kbar_blk;   // Kbar in the block order of the assembly plan (kbar[ab_elems[i]])
   DevBuf<uint8_t> isbc;
   DevBuf<double> stage;   // nv_g doubles: caller-numbered staging for set/get
   DevBuf<double> stage2;  // 2 nv_g (interleaved flux)
@@ -193,8 +192,6 @@ static void compute_kbar(shakti_model* m) {
   ensure_rules(m);
   launch_kbar(m->hm.ne, m->c0.p, m->c1.p, m->c2.p, m->x.p, m->y.p, m->b.p, m->qx.p, m->qy.p, m->kbar.p,
               m->dprm, m->stream);
-  // block-ordered copy for the row-block assembly: its cells then read Kbar without the cell-id indirection
-  if (m->kbar_blk.n) launch_gather((int64_t)m->kbar_blk.n, m->ab_elems.p, m->kbar.p, m->kbar_blk.p, m->stream);
 }
 
 // residual (+ Jacobian) at the current state; Kbar must be current
@@ -206,8 +203,8 @@ static void assemble(shakti_model* m, double dt, int want_J) {
   if (m->opt.assembly_kernel == 0 && m->ab.ok) {
     AssemblyPlanView pl{no, m->ab.rows_per_block, m->ab.n_blocks, m->ab.max_cells, m->ab.max_verts, m->ab_eptr.p,
                         m->ab_elems.p, m->ab_lv.p, m->ab_hptr.p, m->ab_halo.p, m->ab_incptr.p, m->ab_inc.p, m->ab_src.p};
-    launch_assemble_blocks(pl, m->fields(), m->kbar.p, m->kbar_blk.n ? m->kbar_blk.p : nullptr, dt, m->N_bdry, m->J.slice_ptr.p, m->F.p, m->J.val.p, want_J,
-                           m->dprm, m->stream);
+    launch_assemble_blocks(pl, m->fields(), m->kbar.p, dt, m->N_bdry, m->J.slice_ptr.p, m->F.p, m->J.val.p, want_J, m->dprm,
+                           m->stream);
     if (want_J) m->J_valid = true;
     return;
   }
@@ -304,7 +301,7 @@ static KrylovResult linear_solve(shakti_model* m, const double* rhs, double* dx,
     PrecFn M;
     if (m->opt.precond == SHAKTI_PC_JACOBI) {
       launch_extract_dinv(no, m->diag_pos.p, m->J.val.p, m->dinv.p, m->stream);
-      M = [m, no](const double* rr, double* z) { launch_pointwise_mul(no, m->dinv.p, rr, 1.0, z, m->stream); };
+      M = [m, no](const double* rr, double* z) { launch_scaled_mul<double>(no, m->dinv.p, rr, 1.0, z, m->stream); };
     } else {
       M = [m, no](const double* rr, double* z) {
         SHAKTI_CUDA(cudaMemcpyAsync(z, rr, sizeof(double) * no, cudaMemcpyDeviceToDevice, m->stream));
@@ -628,7 +625,6 @@ static void create(int64_t nv, int64_t ne, const double* xy, const int32_t* cell
   if (m->ab.ok) {
     m->ab_eptr.upload(m->ab.blk_eptr);
     m->ab_elems.upload(m->ab.blk_elems);
-    m->kbar_blk.alloc_zero(m->ab.blk_elems.size(), m->stream);
     m->ab_incptr.upload(m->ab.inc_ptr);
     m->ab_inc.upload(m->ab.inc_code);
     m->ab_src.upload(m->ab.src);

@@ -74,9 +74,8 @@ struct AssemblyPlanView {   // device arrays of prep.h AssemblyBlocks
   const uint16_t* inc_code;
   const uint32_t* src;
 };
-// kbar: per cell; kbar_blk: the same values in the plan's block order (kbar[blk_elems[i]]; NULL: not available)
-void launch_assemble_blocks(const AssemblyPlanView& plan, FieldPtrs f, const double* kbar, const double* kbar_blk, double dt,
-                            double N_bdry, const int32_t* slice_ptr, double* F, double* Jval, int want_J, DevParams p, cudaStream_t s);
+void launch_assemble_blocks(const AssemblyPlanView& plan, FieldPtrs f, const double* kbar, double dt, double N_bdry,
+                            const int32_t* slice_ptr, double* F, double* Jval, int want_J, DevParams p, cudaStream_t s);
 void launch_apply_bc(int32_t n_owned, const uint8_t* isbc, const double* N, double N_bdry,
                      const int32_t* diag_pos, double* F, double* Jval, int want_J, cudaStream_t s);
 
@@ -156,8 +155,6 @@ void launch_combine(int64_t n, int nvec, const double* V, int64_t ld, const doub
 void launch_readback(const double* src, double* dst_host, int count, cudaStream_t s);
 void launch_axpy(int64_t n, double alpha, const double* x, double* y, cudaStream_t s);  // y += alpha x
 void launch_xmy_masked(int64_t n, const double* a, const uint8_t* mask, double* out, cudaStream_t s);
-void launch_pointwise_mul(int64_t n, const double* a, const double* b, double scale, double* out, cudaStream_t s);
-void launch_fill(int64_t n, double v, double* x, cudaStream_t s);
 void launch_gather(int64_t n, const int32_t* idx, const double* src, double* dst, cudaStream_t s);   // dst[i] = src[idx[i]]
 void launch_scatter(int64_t n, const int32_t* idx, const double* src, double* dst, cudaStream_t s);  // dst[idx[i]] = src[i]
 // model_setup data ingestion on the device (reference model_setup.py:68-91)

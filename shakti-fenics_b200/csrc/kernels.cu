@@ -562,248 +562,11 @@ assemble_blocks_kernel(int32_t n_owned, int32_t rows_per_block, int32_t cap, int
   }
 }
 
-// ---- version 2 of the row-block kernel (default).  Same algorithm and same plan; what changed, guided by the
-// round-1 ncu capture (issue/latency bound at 24 % occupancy, IMAD+ISETP over half of the stall samples):
-//   * CAP / VCAP are template constants: every shared-memory address is base + immediate, the runtime
-//     multiplications (IMAD) of the 36 vertex loads and 12 stores per cell disappear;
-//   * phase 0 stages the block's OWN rows -- twelve contiguous 1 KB slices -- with the bulk asynchronous copy
-//     engine (cp.async.bulk global -> shared, completion on an mbarrier: SASS UBLKCP), issued by one thread
-//     while the others gather the few halo vertices and prefetch the cell metadata;
-//   * the head is formed per cell from the staged h0 and N (3 FMAs) instead of in the staging pass;
-//   * cells without lake storage (all of them outside the lakes) skip the storage part of the quadrature.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-               "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-
-enum { WX = 0, WY, WH0, WN, WNN, WB, WQX, WQY, WG, WM, WS, WI, WFIELDS };
-
-template <int VCAP>
-__device__ __forceinline__ void element_FJ_staged2(const int v[3], const double* __restrict__ sV, double kb, double dt,
-                                                   const DevParams& p, ElemOut& o, double Nv[3]) {
-  const Geo g = geometry(sV[WX * VCAP + v[0]], sV[WY * VCAP + v[0]], sV[WX * VCAP + v[1]], sV[WY * VCAP + v[1]],
-                         sV[WX * VCAP + v[2]], sV[WY * VCAP + v[2]]);
-  double h[3], bb[3], mm[3], qxv[3], qyv[3], Nn[3], st[3], Gv[3], inp[3];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    Nv[i] = sV[WN * VCAP + v[i]];
-    h[i] = sV[WH0 * VCAP + v[i]] - Nv[i] * p.inv_rwg;   // Head (constitutive.py:6-9)
-    Nn[i] = sV[WNN * VCAP + v[i]];
-    bb[i] = sV[WB * VCAP + v[i]];
-    qxv[i] = sV[WQX * VCAP + v[i]];
-    qyv[i] = sV[WQY * VCAP + v[i]];
-    Gv[i] = sV[WG * VCAP + v[i]];
-    mm[i] = sV[WM * VCAP + v[i]];
-    st[i] = sV[WS * VCAP + v[i]];
-    inp[i] = sV[WI * VCAP + v[i]];
-  }
-  element_core(g, h, bb, mm, qxv, qyv, Nv, Nn, st, Gv, inp, kb, dt, p, o);
-}
-
-template <int CAP, int VCAP>
-__global__ void __launch_bounds__(128, 4)
-assemble_blocks_v2_kernel(int32_t n_owned, int32_t rows_per_block, const int32_t* __restrict__ blk_eptr,
-                          const uint16_t* __restrict__ blk_lv,
-                          const int32_t* __restrict__ blk_hptr, const int32_t* __restrict__ blk_halo,
-                          const int32_t* __restrict__ inc_ptr, const uint16_t* __restrict__ inc_code,
-                          const uint32_t* __restrict__ src, FieldPtrs f, const double* __restrict__ kbar_blk, double dt,
-                          double N_bdry, const int32_t* __restrict__ slice_ptr, double* __restrict__ F,
-                          double* __restrict__ Jval, int want_J, DevParams p) {
-  extern __shared__ __align__(16) double smem[];
-  double* sV = smem;                               // [WFIELDS][VCAP]
-  double* sK = smem + (size_t)WFIELDS * VCAP;      // [12][CAP]: F0..F2, J00..J22
-  uint64_t& bar = *reinterpret_cast<uint64_t*>(sK + (size_t)12 * CAP);   // mbarrier of the bulk copies
-  uint8_t* sBC = reinterpret_cast<uint8_t*>(sK + (size_t)12 * CAP + 1);   // [VCAP]
-  const int32_t r0 = blockIdx.x * rows_per_block;
-  const int32_t nrows = min(rows_per_block, n_owned - r0);
-  const int32_t h0 = blk_hptr[blockIdx.x], nh = blk_hptr[blockIdx.x + 1] - h0;
-  const double* const fld[WFIELDS] = {f.x, f.y, f.h0, f.N, f.N_n, f.b, f.qx, f.qy, f.G, f.melt, f.storage, f.inputs};
-  // ---- phase 0a: own rows by bulk copy (whole blocks only: sizes must be multiples of 16 bytes)
-  const bool bulk = (nrows == rows_per_block) && ((rows_per_block & 1) == 0);
-  if (bulk && threadIdx.x == 0) {
-    mbar_init(&bar, 1);
-    mbar_expect_tx(&bar, (uint32_t)(WFIELDS * nrows * sizeof(double)));
-#pragma unroll
-    for (int k = 0; k < WFIELDS; ++k) bulk_g2s(sV + k * VCAP, fld[k] + r0, (uint32_t)(nrows * sizeof(double)), &bar);
-  }
-  // Kbar (already in block order: no cell-id indirection) and the block-local vertex ids of this thread's
-  // cells are requested first, so that their latency overlaps the staging
-  constexpr int kCellsPre = 4;
-  const int32_t e0 = blk_eptr[blockIdx.x], e1 = blk_eptr[blockIdx.x + 1];
-  double kb_pre[kCellsPre];
-  uint32_t lv01_pre[kCellsPre], lv2_pre[kCellsPre];
-#pragma unroll
-  for (int c = 0; c < kCellsPre; ++c) {
-    const int32_t le = threadIdx.x + c * blockDim.x;
-    kb_pre[c] = 0.0; lv01_pre[c] = 0; lv2_pre[c] = 0;
-    if (le < e1 - e0) {
-      const uint16_t* lv = blk_lv + 3 * (size_t)(e0 + le);
-      lv01_pre[c] = (uint32_t)lv[0] | ((uint32_t)lv[1] << 16);
-      lv2_pre[c] = lv[2];
-      kb_pre[c] = kbar_blk[e0 + le];
-    }
-  }
-  // ---- phase 0b: halo vertices (and everything, for the last partial block) by per-thread loads
-  for (int32_t i = (bulk ? nrows : 0) + threadIdx.x; i < nrows + nh; i += blockDim.x) {
-    const int32_t g = i < nrows ? r0 + i : blk_halo[h0 + i - nrows];
-#pragma unroll
-    for (int k = 0; k < WFIELDS; ++k) sV[k * VCAP + i] = fld[k][g];
-    sBC[i] = f.isbc[g];
-  }
-  if (bulk)
-    for (int32_t i = threadIdx.x; i < nrows; i += blockDim.x) sBC[i] = f.isbc[r0 + i];
-  __syncthreads();            // mbarrier initialised (thread 0) and the per-thread stores are visible
-  if (bulk) mbar_wait(&bar, 0);
-  // ---- phase 1
-#pragma unroll 1
-  for (int c = 0; c * (int32_t)blockDim.x + (int32_t)threadIdx.x < e1 - e0; ++c) {
-    const int32_t le = threadIdx.x + c * blockDim.x;
-    int v[3];
-    double kb;
-    if (c < kCellsPre) {
-      uint32_t a01 = lv01_pre[0], a2 = lv2_pre[0];
-      kb = kb_pre[0];
-#pragma unroll
-      for (int q = 1; q < kCellsPre; ++q)
-        if (c == q) { a01 = lv01_pre[q]; a2 = lv2_pre[q]; kb = kb_pre[q]; }
-      v[0] = a01 & 0xFFFFu; v[1] = a01 >> 16; v[2] = a2;
-    } else {
-      const uint16_t* lv = blk_lv + 3 * (size_t)(e0 + le);
-      v[0] = lv[0]; v[1] = lv[1]; v[2] = lv[2];
-      kb = kbar_blk[e0 + le];
-    }
-    ElemOut o;
-    double Nv[3];
-    element_FJ_staged2<VCAP>(v, sV, kb, dt, p, o, Nv);
-    const bool bc[3] = {sBC[v[0]] != 0, sBC[v[1]] != 0, sBC[v[2]] != 0};
-    apply_lifting(o, Nv, bc, N_bdry);
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-      sK[a * CAP + le] = o.F[a];
-#pragma unroll
-      for (int b = 0; b < 3; ++b) sK[(3 + 3 * a + b) * CAP + le] = (bc[a] || bc[b]) ? 0.0 : o.J[a][b];
-    }
-  }
-  // ---- phase 2 (first loads issued before the barrier, see the version above)
-  constexpr int kPre = 8, kIncPre = 8;
-  uint16_t incpre[kIncPre];
-  const bool has_row = (int32_t)threadIdx.x < nrows;
-  const int32_t row = r0 + threadIdx.x;
-  int32_t base = 0, w = 0, ib = 0, ie = 0;
-  uint32_t pre[kPre];
-  if (has_row) {
-    const int32_t slice = row >> 5;
-    base = slice_ptr[slice];
-    w = (slice_ptr[slice + 1] - base) >> 5;
-    ib = inc_ptr[row];
-    ie = inc_ptr[row + 1];
-#pragma unroll
-    for (int k = 0; k < kIncPre; ++k) incpre[k] = ib + k < ie ? inc_code[ib + k] : (uint16_t)0xFFFFu;
-    if (want_J) {
-#pragma unroll
-      for (int k = 0; k < kPre; ++k) pre[k] = k < w ? src[base + 32 * k + (row & 31)] : 0xFFFFFFFFu;
-    }
-  }
-  __syncthreads();
-  if (!has_row) return;
-  const bool rbc = sBC[threadIdx.x] != 0;
-  double Fr = 0.0, Jd = 0.0;
-#pragma unroll
-  for (int k = 0; k < kIncPre; ++k) {
-    const uint32_t code = incpre[k];
-    if (code != 0xFFFFu) {
-      const uint32_t le = code >> 2, a = code & 3u;
-      Fr += sK[a * CAP + le];
-      Jd += sK[(3 + 4 * a) * CAP + le];
-    }
-  }
-  for (int32_t k = ib + kIncPre; k < ie; ++k) {   // vertices of valence > kIncPre
-    const uint32_t code = inc_code[k];
-    const uint32_t le = code >> 2, a = code & 3u;
-    Fr += sK[a * CAP + le];
-    Jd += sK[(3 + 4 * a) * CAP + le];
-  }
-  F[row] = rbc ? sV[WN * VCAP + threadIdx.x] - N_bdry : Fr;
-  if (!want_J) return;
-  auto entry = [&](uint32_t s2, int32_t pos) {
-    if (s2 == 0xFFFFFFFFu) return;         // padding
-    double v;
-    if (s2 == 0xFFFEFFFEu) v = rbc ? 1.0 : Jd;
-    else {
-      const uint32_t ca = s2 & 0xFFFFu, cb = s2 >> 16;
-      v = sK[(3 + (ca & 15u)) * CAP + (ca >> 4)];
-      if (cb != 0xFFFFu) v += sK[(3 + (cb & 15u)) * CAP + (cb >> 4)];
-    }
-    Jval[pos] = v;
-  };
-#pragma unroll
-  for (int k = 0; k < kPre; ++k)
-    if (k < w) entry(pre[k], base + 32 * k + (row & 31));
-  for (int k = kPre; k < w; ++k) {
-    const int32_t pos = base + 32 * k + (row & 31);
-    entry(src[pos], pos);
-  }
-}
-
-template <int CAP, int VCAP>
-static void launch_assemble_blocks_v2(const AssemblyPlanView& pl, FieldPtrs f, const double* kbar_blk, double dt, double N_bdry,
-                                      const int32_t* slice_ptr, double* F, double* Jval, int want_J, DevParams p, int dev,
-                                      cudaStream_t s) {
-  constexpr size_t smem = ((size_t)WFIELDS * VCAP + (size_t)12 * CAP + 1) * sizeof(double) + VCAP;
-  static bool configured[64] = {};   // the opt-in is per device
-  if (!configured[dev & 63]) {
-    SHAKTI_CUDA(cudaFuncSetAttribute((assemble_blocks_v2_kernel<CAP, VCAP>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    SHAKTI_CUDA(cudaFuncSetAttribute((assemble_blocks_v2_kernel<CAP, VCAP>), cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    configured[dev & 63] = true;
-  }
-  SHAKTI_LAUNCH((assemble_blocks_v2_kernel<CAP, VCAP>), pl.n_blocks, 128, smem, s, pl.n_owned, pl.rows_per_block, pl.blk_eptr,
-                pl.blk_lv, pl.blk_hptr, pl.blk_halo, pl.inc_ptr, pl.inc_code, pl.src, f, kbar_blk, dt, N_bdry, slice_ptr, F,
-                Jval, want_J, p);
-}
-
-void launch_assemble_blocks(const AssemblyPlanView& pl, FieldPtrs f, const double* kbar, const double* kbar_blk, double dt,
-                            double N_bdry, const int32_t* slice_ptr, double* F, double* Jval, int want_J, DevParams p, cudaStream_t s) {
+void launch_assemble_blocks(const AssemblyPlanView& pl, FieldPtrs f, const double* kbar, double dt, double N_bdry,
+                            const int32_t* slice_ptr, double* F, double* Jval, int want_J, DevParams p, cudaStream_t s) {
   if (pl.n_blocks == 0) return;
   int dev = 0;
   SHAKTI_CUDA(cudaGetDevice(&dev));
-  // v2 (compile-time strides, bulk-copy staging) executes 8 % fewer instructions but measured SLOWER at C4
-  // (2.31-2.53 ms vs 2.21 ms, profiles/r2_assembly.md), so it is opt-in: SHAKTI_ASM_V2=1
-  static const bool use_v1 = getenv("SHAKTI_ASM_V2") == nullptr;
-  if (!use_v1 && kbar_blk && pl.rows_per_block == 128) {
-    // compile-time capacities: (350, 226) keeps 4 blocks per SM (55.5 KB each) and covers Morton-ordered
-    // triangulations of structured-like density (C2-C5: at most 350 cells, 226 vertices per block);
-    // (400, 256) is the roomier instance (3 blocks per SM); anything larger runs the runtime-stride kernel
-    if (pl.cap <= 350 && pl.vcap <= 226) {
-      launch_assemble_blocks_v2<350, 226>(pl, f, kbar_blk, dt, N_bdry, slice_ptr, F, Jval, want_J, p, dev, s);
-      return;
-    }
-    if (pl.cap <= 400 && pl.vcap <= 256) {
-      launch_assemble_blocks_v2<400, 256>(pl, f, kbar_blk, dt, N_bdry, slice_ptr, F, Jval, want_J, p, dev, s);
-      return;
-    }
-  }
   const size_t smem = ((size_t)VFIELDS * pl.vcap + (size_t)12 * pl.cap) * sizeof(double) + pl.vcap;
   static size_t configured[64] = {};    // per device (a process may drive several GPUs)
   if (smem > configured[dev & 63]) {
@@ -852,34 +615,6 @@ __device__ __forceinline__ void cell_grad(const WinGeo& w, const double f[3], do
   gy = f[0] * w.g.gy[0] + f[1] * w.g.gy[1] + f[2] * w.g.gy[2];
 }
 
-// q <- -|b|^3 g grad h / (12 nu (1 + omega |q_old|/nu))        (solvers.py:143,186)
-__global__ void __launch_bounds__(256)
-update_q_kernel(int32_t n_owned, const int32_t* __restrict__ win, const double* __restrict__ x,
-                const double* __restrict__ y, const double* __restrict__ h0, const double* __restrict__ N,
-                const double* __restrict__ b, double* __restrict__ qx, double* __restrict__ qy, DevParams p) {
-  const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_owned) return;
-  const WinGeo w = win_geometry(win, i, x, y);
-  if (w.loc < 0) return;
-  double h[3];
-#pragma unroll
-  for (int a = 0; a < 3; ++a) h[a] = h0[w.v[a]] - N[w.v[a]] / p.rwg;
-  double ghx, ghy;
-  cell_grad(w, h, ghx, ghy);
-  const double bi = fabs(b[i]);
-  const double qxo = qx[i], qyo = qy[i];
-  const double Re = sqrt(qxo * qxo + qyo * qyo) / p.nu;
-  const double p1 = -(bi * bi * bi) * p.g;
-  const double p2 = 12.0 * p.nu * (1.0 + p.omega * Re);
-  qx[i] = p1 * ghx / p2;
-  qy[i] = p1 * ghy / p2;
-}
-void launch_update_q(int32_t n_owned, const int32_t* win, const double* x, const double* y, const double* h0,
-                     const double* N, const double* b, double* qx, double* qy, DevParams p, cudaStream_t s) {
-  if (n_owned == 0) return;
-  SHAKTI_LAUNCH(update_q_kernel, div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b, qx, qy, p);
-}
-
 __device__ __forceinline__ double melt_at_vertex(const WinGeo& w, int32_t i, const double* __restrict__ h0,
                                                  const double* __restrict__ N, const double* __restrict__ b,
                                                  const double* __restrict__ qx, const double* __restrict__ qy,
@@ -900,27 +635,6 @@ __device__ __forceinline__ double melt_at_vertex(const WinGeo& w, int32_t i, con
   const double m0 = (G[i] - p.rwg * (qx[i] * ghx + qy[i] * ghy)) / p.Lh;
   const double md = (gb2 * melt[i] + b[i] * (gmx * gbx + gmy * gby)) / (1.0 + gb2);
   return m0 + md;
-}
-
-// melt_n <- Melt(q_new, Head(N_new), G, b_old, melt_old)        (solvers.py:165,189)
-__global__ void __launch_bounds__(256)
-update_melt_kernel(int32_t n_owned, const int32_t* __restrict__ win, const double* __restrict__ x,
-                   const double* __restrict__ y, const double* __restrict__ h0, const double* __restrict__ N,
-                   const double* __restrict__ b, const double* __restrict__ qx, const double* __restrict__ qy,
-                   const double* __restrict__ G, const double* __restrict__ melt_old,
-                   double* __restrict__ melt_new, DevParams p) {
-  const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_owned) return;
-  const WinGeo w = win_geometry(win, i, x, y);
-  if (w.loc < 0) { melt_new[i] = melt_old[i]; return; }
-  melt_new[i] = melt_at_vertex(w, i, h0, N, b, qx, qy, G, melt_old, p);
-}
-void launch_update_melt(int32_t n_owned, const int32_t* win, const double* x, const double* y, const double* h0,
-                        const double* N, const double* b, const double* qx, const double* qy, const double* G,
-                        const double* melt_old, double* melt_new, DevParams p, cudaStream_t s) {
-  if (n_owned == 0) return;
-  SHAKTI_LAUNCH(update_melt_kernel, div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b, qx, qy, G,
-                melt_old, melt_new, p);
 }
 
 // b <- max(b + dt (Melt(q_new, N_new, b_old, melt_new)/rho_i - A b N |N|^(n-1)), b_min)
@@ -952,10 +666,14 @@ void launch_update_b(int32_t n_owned, const int32_t* win, const double* x, const
                 melt, b_new, dt, b_min, p);
 }
 
-// Fused pass 1 of the nodal updates: q and melt_n in one kernel (solvers.py:186,189).  The melt update at
-// vertex i needs the NEW flux at i only, so both come from one load of the winning cell, one geometry
-// and one head gradient.  (The gap-height update needs the new melt at the cell's other vertices and
-// therefore stays a second pass.)
+// Pass 1 of the nodal updates (solvers.py:186,189):
+//   q      <- -|b|^3 g grad h / (12 nu (1 + omega |q_old|/nu))        (solvers.py:143)
+//   melt_n <- Melt(q_new, Head(N_new), G, b_old, melt_old)             (solvers.py:165)
+// Q / MELT select the outputs; with Q false, q is read from memory.  The melt update at vertex i needs the NEW
+// flux at i only, so with both on they come from one load of the winning cell, one geometry and one head
+// gradient.  (The gap-height update needs the new melt at the cell's other vertices and therefore stays a
+// second pass.)
+template <bool Q, bool MELT>
 __global__ void __launch_bounds__(256)
 update_q_melt_kernel(int32_t n_owned, const int32_t* __restrict__ win, const double* __restrict__ x,
                      const double* __restrict__ y, const double* __restrict__ h0, const double* __restrict__ N,
@@ -965,13 +683,16 @@ update_q_melt_kernel(int32_t n_owned, const int32_t* __restrict__ win, const dou
   const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_owned) return;
   const WinGeo w = win_geometry(win, i, x, y);
-  if (w.loc < 0) { melt_new[i] = melt_old[i]; return; }
-  double h[3], bb[3], mm[3];
+  if (w.loc < 0) {
+    if (MELT) melt_new[i] = melt_old[i];
+    return;
+  }
+  double h[3], bb[3], mm[3] = {0.0, 0.0, 0.0};
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
     h[a] = h0[w.v[a]] - N[w.v[a]] / p.rwg;
     bb[a] = b[w.v[a]];
-    mm[a] = melt_old[w.v[a]];
+    if (MELT) mm[a] = melt_old[w.v[a]];
   }
   double ghx, ghy, gbx, gby, gmx, gmy;
   cell_grad(w, h, ghx, ghy);
@@ -980,25 +701,43 @@ update_q_melt_kernel(int32_t n_owned, const int32_t* __restrict__ win, const dou
   // the vertex's own values are those of its slot in the winning cell
   const double b_i = w.loc == 0 ? bb[0] : (w.loc == 1 ? bb[1] : bb[2]);
   const double m_i = w.loc == 0 ? mm[0] : (w.loc == 1 ? mm[1] : mm[2]);
-  const double bi = fabs(b_i);
-  const double qxo = qx[i], qyo = qy[i];
-  const double Re = sqrt(qxo * qxo + qyo * qyo) / p.nu;
-  const double p1 = -(bi * bi * bi) * p.g;
-  const double p2 = 12.0 * p.nu * (1.0 + p.omega * Re);
-  const double qxn = p1 * ghx / p2, qyn = p1 * ghy / p2;
-  qx[i] = qxn;
-  qy[i] = qyn;
+  double qxn = qx[i], qyn = qy[i];
+  if (Q) {
+    const double bi = fabs(b_i);
+    const double Re = sqrt(qxn * qxn + qyn * qyn) / p.nu;
+    const double p1 = -(bi * bi * bi) * p.g;
+    const double p2 = 12.0 * p.nu * (1.0 + p.omega * Re);
+    qxn = p1 * ghx / p2;
+    qyn = p1 * ghy / p2;
+    qx[i] = qxn;
+    qy[i] = qyn;
+  }
+  if (!MELT) return;
   const double gb2 = gbx * gbx + gby * gby;
   const double m0 = (G[i] - p.rwg * (qxn * ghx + qyn * ghy)) / p.Lh;
   const double md = (gb2 * m_i + b_i * (gmx * gbx + gmy * gby)) / (1.0 + gb2);
   melt_new[i] = m0 + md;
 }
+void launch_update_q(int32_t n_owned, const int32_t* win, const double* x, const double* y, const double* h0,
+                     const double* N, const double* b, double* qx, double* qy, DevParams p, cudaStream_t s) {
+  if (n_owned == 0) return;
+  SHAKTI_LAUNCH((update_q_melt_kernel<true, false>), div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b, qx, qy,
+                nullptr, nullptr, nullptr, p);
+}
+void launch_update_melt(int32_t n_owned, const int32_t* win, const double* x, const double* y, const double* h0,
+                        const double* N, const double* b, const double* qx, const double* qy, const double* G,
+                        const double* melt_old, double* melt_new, DevParams p, cudaStream_t s) {
+  if (n_owned == 0) return;
+  // with Q false the kernel only reads qx, qy
+  SHAKTI_LAUNCH((update_q_melt_kernel<false, true>), div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b,
+                const_cast<double*>(qx), const_cast<double*>(qy), G, melt_old, melt_new, p);
+}
 void launch_update_q_melt(int32_t n_owned, const int32_t* win, const double* x, const double* y, const double* h0,
                           const double* N, const double* b, double* qx, double* qy, const double* G,
                           const double* melt_old, double* melt_new, DevParams p, cudaStream_t s) {
   if (n_owned == 0) return;
-  SHAKTI_LAUNCH(update_q_melt_kernel, div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b, qx, qy, G,
-                melt_old, melt_new, p);
+  SHAKTI_LAUNCH((update_q_melt_kernel<true, true>), div_up(n_owned, 256), 256, 0, s, n_owned, win, x, y, h0, N, b, qx, qy,
+                G, melt_old, melt_new, p);
 }
 
 // ------------------------------------------------------------------ SELL-32 SpMV family
@@ -1094,14 +833,14 @@ __global__ void f2d_kernel(int64_t n, const float* __restrict__ a, double* __res
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = (double)a[i];
 }
-static int conv_blocks(int64_t n) { return (int)std::min<int64_t>(148 * 16, std::max<int64_t>(1, (n + 255) / 256)); }
+static int stream_blocks(int64_t n) { return (int)std::min<int64_t>(148 * 16, std::max<int64_t>(1, (n + 255) / 256)); }
 void launch_d2f(int64_t n, const double* a, float* out, cudaStream_t s) {
   if (n == 0) return;
-  SHAKTI_LAUNCH(d2f_kernel, conv_blocks(n), 256, 0, s, n, a, out);
+  SHAKTI_LAUNCH(d2f_kernel, stream_blocks(n), 256, 0, s, n, a, out);
 }
 void launch_f2d(int64_t n, const float* a, double* out, cudaStream_t s) {
   if (n == 0) return;
-  SHAKTI_LAUNCH(f2d_kernel, conv_blocks(n), 256, 0, s, n, a, out);
+  SHAKTI_LAUNCH(f2d_kernel, stream_blocks(n), 256, 0, s, n, a, out);
 }
 __global__ void __launch_bounds__(256)
 sell_scale_to_half_kernel(SellView A, const double* __restrict__ dinv, __half* __restrict__ out) {
@@ -1130,7 +869,7 @@ __global__ void scaled_mul_kernel(int64_t n, const T* __restrict__ a, const T* _
 }
 template <class T> void launch_scaled_mul(int64_t n, const T* a, const T* b, double scale, T* out, cudaStream_t s) {
   if (n == 0) return;
-  SHAKTI_LAUNCH((scaled_mul_kernel<T>), conv_blocks(n), 256, 0, s, n, a, b, (T)scale, out);
+  SHAKTI_LAUNCH((scaled_mul_kernel<T>), stream_blocks(n), 256, 0, s, n, a, b, (T)scale, out);
 }
 template void launch_scaled_mul<double>(int64_t, const double*, const double*, double, double*, cudaStream_t);
 template void launch_scaled_mul<float>(int64_t, const float*, const float*, double, float*, cudaStream_t);
@@ -1142,7 +881,7 @@ __global__ void fill_t_kernel(int64_t n, T v, T* __restrict__ x) {
 }
 template <class T> void launch_fill_t(int64_t n, T v, T* x, cudaStream_t s) {
   if (n == 0) return;
-  SHAKTI_LAUNCH((fill_t_kernel<T>), conv_blocks(n), 256, 0, s, n, v, x);
+  SHAKTI_LAUNCH((fill_t_kernel<T>), stream_blocks(n), 256, 0, s, n, v, x);
 }
 template void launch_fill_t<double>(int64_t, double, double*, cudaStream_t);
 template void launch_fill_t<float>(int64_t, float, float*, cudaStream_t);
@@ -1347,7 +1086,6 @@ static void combine_chunk(int c, int blocks, int64_t n, const double* V, int64_t
     default: SHAKTI_LAUNCH((combine_kernel<8, MODE>), blocks, 256, 0, s, n, V, ld, h, w, scale); break;
   }
 }
-static int stream_blocks(int64_t n) { return (int)std::min<int64_t>(148 * 16, std::max<int64_t>(1, (n + 255) / 256)); }
 
 void launch_multi_axpy_neg(int64_t n, int nvec, const double* V, int64_t ld, const double* h, double* w,
                            cudaStream_t s) {
@@ -1380,11 +1118,6 @@ __global__ void readback_kernel(const double* __restrict__ src, double* __restri
 }
 void launch_readback(const double* src, double* dst_host, int count, cudaStream_t s) {
   if (count <= 0) return;
-  const char* mode = getenv("SHAKTI_READBACK");   // "memcpy": copy engine (A/B switch, read per call)
-  if (mode && mode[0] == 'm' && mode[1] == 'e') {
-    SHAKTI_CUDA(cudaMemcpyAsync(dst_host, src, sizeof(double) * count, cudaMemcpyDeviceToHost, s));
-    return;
-  }
   SHAKTI_LAUNCH(readback_kernel, 1, 64, 0, s, src, dst_host, count);
 }
 
@@ -1473,23 +1206,6 @@ __global__ void xmy_masked_kernel(int64_t n, const double* __restrict__ a, const
 void launch_xmy_masked(int64_t n, const double* a, const uint8_t* mask, double* out, cudaStream_t s) {
   if (n == 0) return;
   SHAKTI_LAUNCH(xmy_masked_kernel, stream_blocks(n), 256, 0, s, n, a, mask, out);
-}
-__global__ void pointwise_mul_kernel(int64_t n, const double* __restrict__ a, const double* __restrict__ b,
-                                     double scale, double* __restrict__ out) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = scale * a[i] * b[i];
-}
-void launch_pointwise_mul(int64_t n, const double* a, const double* b, double scale, double* out, cudaStream_t s) {
-  if (n == 0) return;
-  SHAKTI_LAUNCH(pointwise_mul_kernel, stream_blocks(n), 256, 0, s, n, a, b, scale, out);
-}
-__global__ void fill_kernel(int64_t n, double v, double* __restrict__ x) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) x[i] = v;
-}
-void launch_fill(int64_t n, double v, double* x, cudaStream_t s) {
-  if (n == 0) return;
-  SHAKTI_LAUNCH(fill_kernel, stream_blocks(n), 256, 0, s, n, v, x);
 }
 __global__ void gather_kernel(int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ src,
                               double* __restrict__ dst) {

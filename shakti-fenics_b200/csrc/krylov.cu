@@ -60,7 +60,7 @@ KrylovResult Gmres::solve(const ApplyFn& A, const PrecFn& M, const AllReduceFn& 
   KrylovResult res;
   std::vector<double> H((size_t)(m_ + 1) * m_, 0.0), cs(m_, 0.0), sn(m_, 0.0), g(m_ + 1, 0.0), y(m_, 0.0), hh(m_ + 2, 0.0);
   double* hbuf = host_status_;    // pinned, m_ + 2 doubles
-  launch_fill(n_, 0.0, x, s_);
+  launch_fill_t<double>(n_, 0.0, x, s_);
   SHAKTI_CUDA(cudaMemcpyAsync(r_.p, b, n_ * sizeof(double), cudaMemcpyDeviceToDevice, s_));
   double bnorm = -1.0, tol = 0.0;
   int total = 0;
@@ -185,11 +185,11 @@ KrylovResult BiCgStab::solve(const ApplyFn& A, const PrecFn& M, const AllReduceF
   auto axpby = [&](double a, const double* xx, double bb, const double* yy, double* out) {
     SHAKTI_LAUNCH(axpby_kernel, sblocks(n_), 256, 0, s_, n_, a, xx, bb, yy, out);
   };
-  launch_fill(n_, 0.0, x, s_);
+  launch_fill_t<double>(n_, 0.0, x, s_);
   SHAKTI_CUDA(cudaMemcpyAsync(r_.p, b, n_ * sizeof(double), cudaMemcpyDeviceToDevice, s_));
   SHAKTI_CUDA(cudaMemcpyAsync(r0_.p, b, n_ * sizeof(double), cudaMemcpyDeviceToDevice, s_));
-  launch_fill(n_, 0.0, p_.p, s_);
-  launch_fill(n_, 0.0, v_.p, s_);
+  launch_fill_t<double>(n_, 0.0, p_.p, s_);
+  launch_fill_t<double>(n_, 0.0, v_.p, s_);
   const double bnorm = std::sqrt(std::max(dot(r_.p, r_.p), 0.0));
   const double tol = std::max(rtol * bnorm, atol);
   double rho = 1, alpha = 1, omega = 1, resid = bnorm;
