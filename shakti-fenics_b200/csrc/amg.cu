@@ -404,11 +404,16 @@ __global__ void amg_dense_apply_kernel(int32_t n, const double* __restrict__ D, 
 
 // ------------------------------------------------------------------ smoother kernels
 // Chebyshev step: r = dinv (b - A x); d = c1 d + c2 r; x_out = x + d
-// KG as in spmv_sell_kernel (kernels.cu): 1 = thread per row, 8 = block per slice for small wide-rowed levels
-template <class T, int KG>
+// KG as in spmv_sell_kernel (kernels.cu): 1 = thread per row, 8 = block per slice for small wide-rowed levels.
+// cf = {c1, c2} in device memory (amg_cheby_coef_kernel), so that a new spectral bound changes no kernel argument.
+// MODE, for the fine level of the mixed-precision cycle (Amg::apply):
+//   CHEBY_X_IS_D  first sweep after amg_cycle_entry_kernel, which wrote the first iterate to x only: the old d is x
+//   CHEBY_EXIT    last sweep of the cycle: z = (double)(x + d_new); d is read, d and x_out are not written
+enum { CHEBY_PLAIN = 0, CHEBY_X_IS_D = 1, CHEBY_EXIT = 2 };
+template <class T, int KG, int MODE = CHEBY_PLAIN>
 __global__ void __launch_bounds__(256)
 amg_cheby_kernel(SellViewT<T> A, const T* __restrict__ dinv, const T* __restrict__ b, const T* __restrict__ x,
-                 T* __restrict__ d, T* __restrict__ x_out, T c1, T c2) {
+                 T* __restrict__ d, T* __restrict__ x_out, const double* __restrict__ cf, double* __restrict__ z) {
   pdl_sync();
   int32_t row;
   T acc = 0;
@@ -439,19 +444,26 @@ amg_cheby_kernel(SellViewT<T> A, const T* __restrict__ dinv, const T* __restrict
     for (int j = 1; j < KG; ++j) acc += psum[j][lane];
   }
   if (row >= A.n_rows) return;
+  const T c1 = (T)cf[0], c2 = (T)cf[1];
   const T r = dinv[row] * (b[row] - acc);
-  const T dn = c1 * d[row] + c2 * r;
+  const T dn = c1 * (MODE == CHEBY_X_IS_D ? x[row] : d[row]) + c2 * r;
+  if (MODE == CHEBY_EXIT) {
+    z[row] = (double)(x[row] + dn);
+    return;
+  }
   d[row] = dn;
   x_out[row] = x[row] + dn;
 }
 constexpr int32_t kChebyWideRowsBelow = 300000;
-template <class T>
-static void launch_cheby(SellViewT<T> A, const T* dinv, const T* b, const T* x, T* d, T* x_out, double c1, double c2, cudaStream_t s) {
+template <class T, int MODE = CHEBY_PLAIN>
+static void launch_cheby(SellViewT<T> A, const T* dinv, const T* b, const T* x, T* d, T* x_out, const double* cf, cudaStream_t s) {
+  static_assert(MODE != CHEBY_EXIT, "the exit sweep writes z: launched by Amg::apply");
   // (a variant interleaving two slices per warp was measured slower: 193 vs 179 ms per step)
   if (A.n_rows < kChebyWideRowsBelow)
-    SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 8>), A.n_slices, 256, 0, s, A, dinv, b, x, d, x_out, (T)c1, (T)c2);
+    SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 8, MODE>), A.n_slices, 256, 0, s, A, dinv, b, x, d, x_out, cf, nullptr);
   else
-    SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 1>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, dinv, b, x, d, x_out, (T)c1, (T)c2);
+    SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 1, MODE>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, dinv, b, x, d, x_out, cf,
+                      nullptr);
 }
 
 // ---- the same two kernels of the LARGE levels on the half-precision, row-scaled copy Ah = D^-1 A (unit
@@ -462,7 +474,7 @@ static void launch_cheby(SellViewT<T> A, const T* dinv, const T* b, const T* x, 
 __global__ void __launch_bounds__(256)
 amg_cheby_h_kernel(int32_t n_rows, int32_t n_slices, const int32_t* __restrict__ slice_ptr, const int32_t* __restrict__ col,
                    const __half* __restrict__ val, const float* __restrict__ dinv, const float* __restrict__ b,
-                   const float* __restrict__ x, float* __restrict__ d, float* __restrict__ x_out, float c1, float c2) {
+                   const float* __restrict__ x, float* __restrict__ d, float* __restrict__ x_out, const double* __restrict__ cf) {
   pdl_sync();
   const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
   const int32_t slice = row >> 5;
@@ -475,6 +487,7 @@ amg_cheby_h_kernel(int32_t n_rows, int32_t n_slices, const int32_t* __restrict__
 #pragma unroll 4
   for (int k = 0; k < w; ++k) acc += __half2float(vp[32 * k]) * x[cp[32 * k]];
   if (row >= n_rows) return;
+  const float c1 = (float)cf[0], c2 = (float)cf[1];
   const float r = dinv[row] * b[row] - acc;
   const float dn = c1 * d[row] + c2 * r;
   d[row] = dn;
@@ -503,34 +516,123 @@ amg_resid_h_kernel(int32_t n_rows, int32_t n_slices, const int32_t* __restrict__
 // does level operator A run on its half-precision copy?
 static bool uses_half(const Amg::Impl& I, const DevSell& A);
 
-// first Chebyshev step from a zero guess: d = (dinv b)/theta ; x = d
+// V-cycle entry on the fine level of the mixed-precision cycle: b = (float)r, and the first Chebyshev step from a
+// zero guess, x = (dinv b)/theta -- the work of d2f_kernel and amg_cheby_first_kernel in one pass.  d is not
+// written: the next sweep reads x in its place (CHEBY_X_IS_D).
+__global__ void amg_cycle_entry_kernel(int32_t n, const double* __restrict__ r, const float* __restrict__ dinv,
+                                       const double* __restrict__ inv_theta, float* __restrict__ b, float* __restrict__ x) {
+  const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float bi = (float)r[i];
+  b[i] = bi;
+  x[i] = dinv[i] * bi * (float)inv_theta[0];
+}
+
+// first Chebyshev step from a zero guess: d = (dinv b)/theta ; x = d   (inv_theta = 1/theta in device memory)
 template <class T>
-__global__ void amg_cheby_first_kernel(int32_t n, const T* __restrict__ dinv, const T* __restrict__ b, T inv_theta,
-                                       T* __restrict__ d, T* __restrict__ x) {
+__global__ void amg_cheby_first_kernel(int32_t n, const T* __restrict__ dinv, const T* __restrict__ b,
+                                       const double* __restrict__ inv_theta, T* __restrict__ d, T* __restrict__ x) {
   pdl_sync();
   const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const T v = dinv[i] * b[i] * inv_theta;
+  const T v = dinv[i] * b[i] * (T)inv_theta[0];
   d[i] = v;
   x[i] = v;
 }
 
-// Gershgorin bound of lambda_max(D^-1 A): max_i |dinv_i| sum_j |a_ij|, reduced with an integer
-// atomicMax on the bit pattern (valid for non-negative doubles)
+// Block maximum of v (256 threads), then one integer atomicMax on the bit pattern (valid for non-negative
+// doubles).  A maximum does not depend on the order of its operands, so the result is the same bits however the
+// rows are split among threads and blocks.
+__device__ __forceinline__ void block_max_to(double v, unsigned long long* __restrict__ out) {
+  __shared__ double wmax[8];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+  if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = v;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int j = 1; j < 8; ++j) v = fmax(v, wmax[j]);
+    if (v > 0.0) atomicMax(out, (unsigned long long)__double_as_longlong(v));
+  }
+}
+// few blocks with a grid-stride loop: one same-address atomic per block (one per warp, 500 000 at 16M rows, took
+// four times as long as streaming the matrix)
+static int bound_blocks(int64_t rows, int sm_count) { return (int)std::min<int64_t>((int64_t)sm_count * 8, std::max<int64_t>(1, div_up(rows, 256))); }
+
+// Gershgorin bound of lambda_max(D^-1 A): max_i |dinv_i| sum_j |a_ij|
 __global__ void __launch_bounds__(256)
 amg_gershgorin_kernel(SellView A, const double* __restrict__ dinv, unsigned long long* __restrict__ out) {
-  const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
   double v = 0.0;
-  if (row < A.n_rows) {
+  for (int32_t row = blockIdx.x * blockDim.x + threadIdx.x; row < A.n_rows; row += gridDim.x * blockDim.x) {
     const int32_t base = A.slice_ptr[row >> 5] + (row & 31);
     const int32_t w = (A.slice_ptr[(row >> 5) + 1] - A.slice_ptr[row >> 5]) >> 5;
     double acc = 0.0;
     for (int k = 0; k < w; ++k) acc += fabs(A.val[base + 32 * k]);
-    v = fabs(dinv[row]) * acc;
+    v = fmax(v, fabs(dinv[row]) * acc);
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-  if ((threadIdx.x & 31) == 0 && v > 0.0) atomicMax(out, (unsigned long long)__double_as_longlong(v));
+  block_max_to(v, out);
+}
+
+// The fine level's smoother refresh in one pass over its fp64 values (mixed-precision cycle, Chebyshev smoother).
+// Per row: the diagonal, picked out by its slot; dinv in fp64 and fp32; the fp32 copy of every stored entry,
+// padding slots and the padding rows of the last slice included (F32 = false: the level runs on its half-precision
+// copy, made afterwards from dinv); and the row's Gershgorin number |dinv_i| sum_j |a_ij|.  Same operations in the
+// same order as amg_dinv_kernel, d2f_kernel and amg_gershgorin_kernel, so the results are the same bits.
+template <bool F32>
+__global__ void __launch_bounds__(256)
+amg_fine_refresh_kernel(SellView A, const int32_t* __restrict__ diag_pos, double* __restrict__ dinv, float* __restrict__ dinvf,
+                        float* __restrict__ valf, unsigned long long* __restrict__ bound) {
+  double v = 0.0;
+  const int32_t rows = A.n_slices * 32;
+  for (int32_t row = blockIdx.x * blockDim.x + threadIdx.x; row < rows; row += gridDim.x * blockDim.x) {
+    const int32_t base = A.slice_ptr[row >> 5] + (row & 31);
+    const int32_t w = (A.slice_ptr[(row >> 5) + 1] - A.slice_ptr[row >> 5]) >> 5;
+    double di = 0.0;
+    if (row < A.n_rows) {
+      const double d = A.val[diag_pos[row]];
+      di = d != 0.0 ? 1.0 / d : 0.0;
+      dinv[row] = di;
+      dinvf[row] = (float)di;
+    }
+    double acc = 0.0;
+#pragma unroll 4
+    for (int k = 0; k < w; ++k) {
+      const double a = A.val[base + 32 * k];
+      if (F32) valf[base + 32 * k] = (float)a;
+      acc += fabs(a);
+    }
+    if (row < A.n_rows) v = fmax(v, fabs(di) * acc);
+  }
+  block_max_to(v, bound);
+}
+
+// Chebyshev coefficients of levels [0, nl) from their bounds of lambda_max(D^-1 A), kept in device memory so that a
+// new bound needs no host round trip and changes no kernel argument of the captured V-cycle.  Per level (stride
+// `stride`): [0] = 1/theta, then sweep k's pair (c1, c2) at [2 + 2k].  A bound that is not positive and finite gives
+// 2.0, or with `keep` leaves the level's previous value.  The formulas and the order of the operations are those the
+// host used; the _rn intrinsics keep the compiler from contracting any of them into a fused multiply-add.
+__global__ void amg_cheby_coef_kernel(int nl, int sweeps, int stride, double ratio, const double* __restrict__ bound, int keep,
+                                      double* __restrict__ lmax, double* __restrict__ coef) {
+  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+  for (int l = 0; l < nl; ++l) {
+    const double h = bound[l];
+    if (h > 0.0 && isfinite(h)) lmax[l] = h;
+    else if (!keep) lmax[l] = 2.0;
+    const double hi = lmax[l], lo = __ddiv_rn(hi, ratio);
+    const double theta = __dmul_rn(0.5, __dadd_rn(hi, lo)), delta = __dmul_rn(0.5, __dsub_rn(hi, lo));
+    const double sigma = __ddiv_rn(theta, delta);
+    double rho = __ddiv_rn(1.0, sigma);
+    double* __restrict__ c = coef + (size_t)l * stride;
+    c[0] = __ddiv_rn(1.0, theta);
+    c[2] = 0.0;    // sweep 0 from a nonzero guess
+    c[3] = c[0];
+    for (int k = 1; k < sweeps; ++k) {
+      const double rho_n = __ddiv_rn(1.0, __dsub_rn(__dmul_rn(2.0, sigma), rho));
+      c[2 + 2 * k] = __dmul_rn(rho_n, rho);
+      c[3 + 2 * k] = __ddiv_rn(__dmul_rn(2.0, rho_n), delta);
+      rho = rho_n;
+    }
+  }
 }
 
 // ------------------------------------------------------------------ distributed helpers
@@ -614,7 +716,7 @@ struct AmgLevel {
   DevBuf<int32_t> tmap;
   CycleVecs<double> vd;       // V-cycle work vectors, double ...
   CycleVecs<float> vf;        // ... or single precision (mixed-precision cycle)
-  double lmax = 2.0;          // estimate of lambda_max(D^-1 A)
+  int32_t index = 0;          // position in the hierarchy
   bool last = false;
   HostCsr hA;                 // host pattern (levels >= 1)
   HostSell hS;
@@ -646,11 +748,17 @@ struct Amg::Impl {
   bool built = false;
   double op_complexity = 0.0;
   Reducer red;
-  DevBuf<double> scal, lmax_dev;
-  double* host_scal = nullptr;
+  // Chebyshev smoother: per level the bound of lambda_max(D^-1 A) being reduced, the value in use and the
+  // coefficients made from it (amg_cheby_coef_kernel; coef_stride doubles per level)
+  DevBuf<double> lmax_bound, lmax, coef;
+  int coef_stride = 0, coef_sweeps = 0;
+  DevBuf<double> fixed_coef;   // {c1, c2} of launch_level_smoother
   // the V-cycle as a CUDA graph: one launch instead of ~100 kernel launches + ~35 NCCL calls
   cudaGraphExec_t gexec = nullptr;
-  bool graph_valid = false;    // false after every change of kernel arguments (refresh)
+  bool graph_valid = false;    // false after a refresh of the hierarchy
+  const void* graph_key[5] = {};   // buffers of the fine matrix the captured graph reads
+  bool graph_seams = false;        // the captured cycle leaves its first and last fine step to Amg::apply
+  const float* exit_x = nullptr;   // seams: the iterate the last fine sweep (amg_cheby_kernel<CHEBY_EXIT>) reads
   bool warm = false;           // one plain cycle after a (re)build so that lazy allocations are done
   int64_t graph_launches = 0;  // kernels inside the graph (for the launch accounting)
   void* result_ptr = nullptr;  // where level 0's solution ends up
@@ -678,7 +786,6 @@ struct Amg::Impl {
   P2pGather tail_gather;             // right-hand side all-gather through the symmetric heap
   DevBuf<double> tail_rhs_d, tail_gather_d;   // NCCL fallback: padded blocks
   ~Impl() {
-    if (host_scal) cudaFreeHost(host_scal);
     if (gexec) cudaGraphExecDestroy(gexec);
   }
 };
@@ -719,8 +826,7 @@ void Amg::setup(const HostCsr& A0, const HostSell& S0, const std::vector<uint8_t
   I.sm_count = sm_count;
   I.tail.reset();
   I.tail_level = -1;
-  I.scal.alloc_zero(4, s);
-  if (!I.host_scal) SHAKTI_CUDA(cudaMallocHost(&I.host_scal, 32 * sizeof(double)));
+  I.fixed_coef.upload(std::vector<double>{0.3, 0.2});
   refreshes_ = 0;
 }
 
@@ -778,45 +884,78 @@ static bool uses_half(const Amg::Impl& I, const DevSell& A) {
 
 // Copies the V-cycle reads: smoother diagonal in the cycle's precision and, for the mixed-precision
 // cycle, single-precision values of A, P and R (half-precision row-scaled values of A on the large levels).
-static void sync_cycle_precision(Amg::Impl& I, size_t l, const DevSell& Afine, bool matrices) {
+// fine_done: level 0's diagonal and A were copied by fine_refresh_pass.
+static void sync_cycle_precision(Amg::Impl& I, size_t l, const DevSell& Afine, bool matrices, bool fine_done = false) {
   cudaStream_t s = I.s;
   AmgLevel& L = *I.lv[l];
   const DevSell& A = (l == 0) ? Afine : L.A;
   if (I.opt.fp32_cycle) {
-    launch_d2f(L.n, L.dinv.p, L.vf.dinv.p, s);
-    if (uses_half(I, A)) A.refresh_f16_scaled(L.dinv.p, s);
-    else A.refresh_f32(s);
+    if (!(l == 0 && fine_done)) {
+      launch_d2f(L.n, L.dinv.p, L.vf.dinv.p, s);
+      if (uses_half(I, A)) A.refresh_f16_scaled(L.dinv.p, s);
+      else A.refresh_f32(s);
+    }
     if (matrices && !L.last) { L.P.refresh_f32(s); L.R.refresh_f32(s); }
   } else if (L.n) {
     SHAKTI_CUDA(cudaMemcpyAsync(L.vd.dinv.p, L.dinv.p, sizeof(double) * L.n, cudaMemcpyDeviceToDevice, s));
   }
 }
 
+// Level 0 takes the one-pass refresh (amg_fine_refresh_kernel) when it needs both what that pass fuses: the
+// copies of the mixed-precision cycle and the Chebyshev bound.
+static bool fine_one_pass(const Amg::Impl& I) { return I.opt.fp32_cycle && I.opt.smoother == 1 && I.lv[0]->n > 0; }
+
+// dinv (fp64, fp32), the cycle's copy of the fine values and level 0's bound (atomic maximum into `bound`, zeroed
+// by the caller) in one pass; the half-precision copy, where level 0 uses one, is made from dinv afterwards
+static void fine_refresh_pass(Amg::Impl& I, const DevSell& Afine, const int32_t* fine_diag_pos, double* bound) {
+  cudaStream_t s = I.s;
+  AmgLevel& L = *I.lv[0];
+  unsigned long long* b = reinterpret_cast<unsigned long long*>(bound);
+  const int grid = bound_blocks((int64_t)Afine.n_slices * 32, I.sm_count);
+  if (uses_half(I, Afine)) {
+    SHAKTI_LAUNCH(amg_fine_refresh_kernel<false>, grid, 256, 0, s, view(Afine), fine_diag_pos, L.dinv.p, L.vf.dinv.p, nullptr, b);
+    Afine.refresh_f16_scaled(L.dinv.p, s);
+  } else {
+    if (Afine.valf.n != (size_t)Afine.padded) Afine.valf.alloc((size_t)Afine.padded);
+    SHAKTI_LAUNCH(amg_fine_refresh_kernel<true>, grid, 256, 0, s, view(Afine), fine_diag_pos, L.dinv.p, L.vf.dinv.p, Afine.valf.p, b);
+  }
+}
+
+static void launch_cheby_coef(Amg::Impl& I, int nl, bool keep) {
+  SHAKTI_LAUNCH(amg_cheby_coef_kernel, 1, 32, 0, I.s, nl, I.coef_sweeps, I.coef_stride, I.opt.cheby_ratio, I.lmax_bound.p,
+                keep ? 1 : 0, I.lmax.p, I.coef.p);
+}
+
 // Upper end of the spectrum of D^-1 A for the Chebyshev smoother, recomputed at every refresh: the
-// Gershgorin number max_i sum_j |a_ij| / |a_ii| -- one pass per level, one host read for all levels,
-// identical on every rank.  It is a guaranteed upper bound.  (Round-1 history: 1.1 x a warm-started
-// power-iteration estimate is ~4 % faster at 16M dofs but under-estimates after large changes of the
-// operator, which makes the smoother amplify the top of the spectrum and stalled the Krylov solve on a
-// small case; a bound cannot do that.)
-static void update_smoother_bounds(Amg::Impl& I, const DevSell& Afine) {
+// Gershgorin number max_i sum_j |a_ij| / |a_ii| -- one pass per level, identical on every rank, turned
+// into the smoother's coefficients on the device.  It is a guaranteed upper bound.  (Round-1 history: 1.1 x
+// a warm-started power-iteration estimate is ~4 % faster at 16M dofs but under-estimates after large changes
+// of the operator, which makes the smoother amplify the top of the spectrum and stalled the Krylov solve on
+// a small case; a bound cannot do that.)  Returns whether level 0 went through fine_refresh_pass.
+static bool update_smoother_bounds(Amg::Impl& I, const DevSell& Afine, const int32_t* fine_diag_pos) {
   cudaStream_t s = I.s;
   const size_t nl = I.lv.size();
-  if (I.opt.smoother != 1) return;
-  if (I.lmax_dev.n < nl) { I.lmax_dev.alloc_zero(std::max<size_t>(nl, 16), s); }
-  SHAKTI_CUDA(cudaMemsetAsync(I.lmax_dev.p, 0, sizeof(double) * nl, s));
+  if (I.opt.smoother != 1) return false;
+  if (I.lmax_bound.n < nl) {
+    // sized once per hierarchy, before the first capture of the V-cycle
+    I.coef_sweeps = std::max({I.opt.presmooth, I.opt.postsmooth, 8});
+    I.coef_stride = 2 + 2 * I.coef_sweeps;
+    I.lmax_bound.alloc_zero(nl, s);
+    I.lmax.alloc_zero(nl, s);
+    I.coef.alloc_zero(nl * I.coef_stride, s);
+  }
+  SHAKTI_CUDA(cudaMemsetAsync(I.lmax_bound.p, 0, sizeof(double) * nl, s));
+  const bool fine = fine_one_pass(I);
   for (size_t l = 0; l < nl; ++l) {
     AmgLevel& L = *I.lv[l];
-    if (L.n > 0)
-      SHAKTI_LAUNCH(amg_gershgorin_kernel, div_up(L.n, 256), 256, 0, s, view(l == 0 ? Afine : L.A), L.dinv.p,
-                    reinterpret_cast<unsigned long long*>(I.lmax_dev.p + l));
+    if (l == 0 && fine) fine_refresh_pass(I, Afine, fine_diag_pos, I.lmax_bound.p);
+    else if (L.n > 0)
+      SHAKTI_LAUNCH(amg_gershgorin_kernel, bound_blocks(L.n, I.sm_count), 256, 0, s, view(l == 0 ? Afine : L.A), L.dinv.p,
+                    reinterpret_cast<unsigned long long*>(I.lmax_bound.p + l));
   }
-  comm_allreduce_max(I.lmax_dev.p, (int)nl, s);
-  std::vector<double> h(nl);
-  SHAKTI_REQUIRE(nl <= 32, "AMG: more than 32 levels");
-  launch_readback(I.lmax_dev.p, I.host_scal, (int)nl, s);
-  SHAKTI_CUDA(cudaStreamSynchronize(s));
-  for (size_t l = 0; l < nl; ++l) h[l] = I.host_scal[l];
-  for (size_t l = 0; l < nl; ++l) I.lv[l]->lmax = (h[l] > 0 && std::isfinite(h[l])) ? h[l] : 2.0;
+  comm_allreduce_max(I.lmax_bound.p, (int)nl, s);
+  launch_cheby_coef(I, (int)nl, false);
+  return fine;
 }
 
 // One coarsening step on the host: rank-local aggregation on strong connections, prolongator
@@ -1020,6 +1159,7 @@ static void coarsen_level(Amg::Impl& I, size_t l, const DevSell& dA, const HostC
   Ln->hA = product_pattern(R, AP);
   Ln->hA.n_cols = (int64_t)nc + gc;
   Ln->hS = sell_from_csr(Ln->hA);
+  Ln->index = (int32_t)l + 1;
   Ln->n = nc;
   Ln->n_ghost = gc;
   Ln->n_cols = nc + gc;
@@ -1268,24 +1408,29 @@ static void build_hierarchy(Amg::Impl& I, const DevSell& Afine, const int32_t* f
 
 // Cheap per-solve update when the hierarchy itself is kept (lagged): the fine-level smoother must
 // match the CURRENT operator, so its diagonal is recomputed and its Chebyshev bound is set to the
-// (always safe) Gershgorin bound.  Coarse levels stay consistent among themselves.
+// (always safe) Gershgorin bound.  Coarse levels stay consistent among themselves.  Everything stays on
+// the device and no kernel argument changes, so the captured V-cycle is replayed as it is.
 void Amg::refresh_fine_smoother(const DevSell& Afine, const int32_t* fine_diag_pos) {
   Impl& I = *p_;
   cudaStream_t s = I.s;
   if (!I.built || I.lv.empty()) return;
-  I.graph_valid = false;
   AmgLevel& L = *I.lv[0];
-  if (L.n > 0) SHAKTI_LAUNCH(amg_dinv_kernel, div_up(L.n, 256), 256, 0, s, L.n, fine_diag_pos, Afine.val.p, L.dinv.p);
-  if (I.opt.smoother != 1 || (L.last && I.dense_coarse)) { sync_cycle_precision(I, 0, Afine, false); return; }
-  SHAKTI_CUDA(cudaMemsetAsync(I.scal.p + 1, 0, sizeof(double), s));
-  if (L.n > 0)
-    SHAKTI_LAUNCH(amg_gershgorin_kernel, div_up(L.n, 256), 256, 0, s, view(Afine), L.dinv.p,
-                  reinterpret_cast<unsigned long long*>(I.scal.p + 1));
-  comm_allreduce_max(I.scal.p + 1, 1, s);
-  launch_readback(I.scal.p + 1, I.host_scal, 1, s);
-  SHAKTI_CUDA(cudaStreamSynchronize(s));
-  if (I.host_scal[0] > 0 && std::isfinite(I.host_scal[0])) L.lmax = I.host_scal[0];
-  sync_cycle_precision(I, 0, Afine, false);
+  const bool cheby = I.opt.smoother == 1 && !(L.last && I.dense_coarse);
+  if (cheby) SHAKTI_CUDA(cudaMemsetAsync(I.lmax_bound.p, 0, sizeof(double), s));
+  const bool fine = cheby && fine_one_pass(I);
+  if (fine) {
+    fine_refresh_pass(I, Afine, fine_diag_pos, I.lmax_bound.p);
+  } else {
+    if (L.n > 0) SHAKTI_LAUNCH(amg_dinv_kernel, div_up(L.n, 256), 256, 0, s, L.n, fine_diag_pos, Afine.val.p, L.dinv.p);
+    if (cheby && L.n > 0)
+      SHAKTI_LAUNCH(amg_gershgorin_kernel, bound_blocks(L.n, I.sm_count), 256, 0, s, view(Afine), L.dinv.p,
+                    reinterpret_cast<unsigned long long*>(I.lmax_bound.p));
+  }
+  if (cheby) {
+    comm_allreduce_max(I.lmax_bound.p, 1, s);
+    launch_cheby_coef(I, 1, true);
+  }
+  sync_cycle_precision(I, 0, Afine, false, fine);
 }
 
 void Amg::refresh(const DevSell& Afine, const int32_t* fine_diag_pos) {
@@ -1297,8 +1442,9 @@ void Amg::refresh(const DevSell& Afine, const int32_t* fine_diag_pos) {
     { SHAKTI_PHASE("rf_numeric", s); for (size_t l = 0; l < I.lv.size(); ++l) numeric_level(I, l, Afine, fine_diag_pos); }
     { SHAKTI_PHASE("rf_tail", s); refresh_tail(I, Afine); }
   }
-  { SHAKTI_PHASE("rf_bounds", s); update_smoother_bounds(I, Afine); }
-  { SHAKTI_PHASE("rf_f32", s); for (size_t l = 0; l < I.lv.size(); ++l) sync_cycle_precision(I, l, Afine, true); }
+  bool fine_done;
+  { SHAKTI_PHASE("rf_bounds", s); fine_done = update_smoother_bounds(I, Afine, fine_diag_pos); }
+  { SHAKTI_PHASE("rf_f32", s); for (size_t l = 0; l < I.lv.size(); ++l) sync_cycle_precision(I, l, Afine, true, fine_done); }
   if (I.dense_coarse) {
     AmgLevel& L = *I.lv.back();
     const DevSell& A = (I.lv.size() == 1) ? Afine : L.A;
@@ -1316,19 +1462,23 @@ void Amg::refresh(const DevSell& Afine, const int32_t* fine_diag_pos) {
   ++refreshes_;
 }
 
+// x_is_d: CHEBY_X_IS_D (never on a level that runs on its half-precision copy: see seams_apply, restrict_starts)
 template <class T>
-static void cheby_step(Amg::Impl& I, const DevSell& A, const T* dinv, const T* b, const T* x, T* d, T* x_out, double c1, double c2,
-                       cudaStream_t s) {
-  launch_cheby<T>(view_as<T>(A), dinv, b, x, d, x_out, c1, c2, s);
+static void cheby_step(Amg::Impl& I, const DevSell& A, const T* dinv, const T* b, const T* x, T* d, T* x_out, const double* cf,
+                       cudaStream_t s, bool x_is_d = false) {
+  if (x_is_d) launch_cheby<T, CHEBY_X_IS_D>(view_as<T>(A), dinv, b, x, d, x_out, cf, s);
+  else launch_cheby<T>(view_as<T>(A), dinv, b, x, d, x_out, cf, s);
 }
 template <>
 void cheby_step<float>(Amg::Impl& I, const DevSell& A, const float* dinv, const float* b, const float* x, float* d, float* x_out,
-                       double c1, double c2, cudaStream_t s) {
-  if (uses_half(I, A))
+                       const double* cf, cudaStream_t s, bool x_is_d) {
+  if (x_is_d)
+    launch_cheby<float, CHEBY_X_IS_D>(viewf(A), dinv, b, x, d, x_out, cf, s);
+  else if (uses_half(I, A))
     SHAKTI_LAUNCH_PDL(amg_cheby_h_kernel, div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A.n_rows, A.n_slices, A.slice_ptr.p, A.col.p,
-                      A.valh.p, dinv, b, x, d, x_out, (float)c1, (float)c2);
+                      A.valh.p, dinv, b, x, d, x_out, cf);
   else
-    launch_cheby<float>(viewf(A), dinv, b, x, d, x_out, c1, c2, s);
+    launch_cheby<float>(viewf(A), dinv, b, x, d, x_out, cf, s);
 }
 template <class T>
 static void level_residual(Amg::Impl& I, const DevSell& A, const T* dinv, const T* x, const T* b, T* r, cudaStream_t s) {
@@ -1345,9 +1495,13 @@ void level_residual<float>(Amg::Impl& I, const DevSell& A, const float* dinv, co
 
 // `sweeps` smoothing steps on A x = b, in place on v.x (ping-pong with v.x2).  zero_guess: v.x is
 // taken as 0 and the first step needs no SpMV.  Every SpMV is preceded by the level's halo exchange
-// unless the caller says the ghosts are already current.
+// unless the caller says the ghosts are already current.  seam (Chebyshev on the fine level, see
+// seams_apply): kSeamEntry -- the zero-guess step was done by amg_cycle_entry_kernel, which left d
+// unwritten; kSeamExit -- the last sweep is left to Amg::apply, which reads I.exit_x.
+enum { kSeamEntry = 1, kSeamExit = 2 };
 template <class T>
-static void smooth(Amg::Impl& I, AmgLevel& L, const DevSell& A, const T* b, int sweeps, bool zero_guess, bool ghosts_current) {
+static void smooth(Amg::Impl& I, AmgLevel& L, const DevSell& A, const T* b, int sweeps, bool zero_guess, bool ghosts_current,
+                   int seam = 0) {
   cudaStream_t s = I.s;
   CycleVecs<T>& v = vecs<T>(L);
   if (sweeps <= 0) {
@@ -1355,25 +1509,22 @@ static void smooth(Amg::Impl& I, AmgLevel& L, const DevSell& A, const T* b, int 
     return;
   }
   if (I.opt.smoother == 1) {   // Chebyshev polynomial of degree `sweeps` on D^-1 A, interval [lmax/ratio, lmax]
-    const double hi = L.lmax, lo = L.lmax / I.opt.cheby_ratio;
-    const double theta = 0.5 * (hi + lo), delta = 0.5 * (hi - lo), sigma = theta / delta;
-    double rho = 1.0 / sigma;
+    // coefficients: amg_cheby_coef_kernel
+    SHAKTI_REQUIRE(sweeps <= I.coef_sweeps, "AMG: more Chebyshev sweeps than coefficients");
+    const double* cf = I.coef.p + (size_t)L.index * I.coef_stride;
     int k0 = 0;
     if (zero_guess) {
-      if (L.n) SHAKTI_LAUNCH_PDL((amg_cheby_first_kernel<T>), div_up(L.n, 256), 256, 0, s, L.n, v.dinv.p, b, (T)(1.0 / theta), v.d.p, v.x.p);
+      if (L.n && !(seam & kSeamEntry))
+        SHAKTI_LAUNCH_PDL((amg_cheby_first_kernel<T>), div_up(L.n, 256), 256, 0, s, L.n, v.dinv.p, b, cf, v.d.p, v.x.p);
       k0 = 1;
     }
     for (int k = k0; k < sweeps; ++k) {
-      double c1, c2;
-      if (k == 0) { c1 = 0.0; c2 = 1.0 / theta; }
-      else {
-        const double rho_n = 1.0 / (2.0 * sigma - rho);
-        c1 = rho_n * rho;
-        c2 = 2.0 * rho_n / delta;
-        rho = rho_n;
-      }
       if (I.opt.smoother_halo && !(ghosts_current && k == k0)) L.halo->exchange(v.x.p, s);
-      if (L.n) cheby_step<T>(I, A, v.dinv.p, b, v.x.p, v.d.p, v.x2.p, c1, c2, s);
+      if ((seam & kSeamExit) && k == sweeps - 1) {
+        I.exit_x = reinterpret_cast<const float*>(v.x.p);
+        break;
+      }
+      if (L.n) cheby_step<T>(I, A, v.dinv.p, b, v.x.p, v.d.p, v.x2.p, cf + 2 + 2 * k, s, (seam & kSeamEntry) && k == k0);
       std::swap(v.x.p, v.x2.p);
     }
   } else {                      // damped Jacobi
@@ -1388,8 +1539,16 @@ static void smooth(Amg::Impl& I, AmgLevel& L, const DevSell& A, const T* b, int 
   }
 }
 
+// Does the restriction onto level c also take c's first smoothing step (launch_restrict_cheby_first)?  For a
+// level smoothed locally by Chebyshev from a zero guess, with a second step to take over the fused start's
+// unwritten d: not the replicated level, not the coarsest level, not a level on its half-precision copy.
+static bool restrict_starts(const Amg::Impl& I, size_t c) {
+  const AmgLevel& C = *I.lv[c];
+  return I.opt.smoother == 1 && I.opt.presmooth >= 2 && !C.last && (int)c != I.tail_level && !uses_half(I, C.A);
+}
+
 template <class T>
-static void vcycle(Amg::Impl& I, const DevSell& Afine) {
+static void vcycle(Amg::Impl& I, const DevSell& Afine, bool seams) {
   cudaStream_t s = I.s;
   const int nl = (int)I.lv.size();
   for (int l = 0; l < nl; ++l) {   // downward; level l's right-hand side is vecs(l).b
@@ -1434,10 +1593,15 @@ static void vcycle(Amg::Impl& I, const DevSell& Afine) {
       }
       break;
     }
-    smooth<T>(I, L, A, v.b.p, I.opt.presmooth, true, false);
+    const bool started = l > 0 && restrict_starts(I, l);
+    smooth<T>(I, L, A, v.b.p, I.opt.presmooth, true, false, (seams && l == 0) || started ? kSeamEntry : 0);
     L.halo->exchange(v.x.p, s);
     level_residual<T>(I, A, v.dinv.p, v.x.p, v.b.p, v.r.p, s);
-    launch_spmv<T>(view_as<T>(L.R), v.r.p, vecs<T>(*I.lv[l + 1]).b.p, s);
+    CycleVecs<T>& vc = vecs<T>(*I.lv[l + 1]);
+    if (restrict_starts(I, l + 1))
+      launch_restrict_cheby_first<T>(view_as<T>(L.R), v.r.p, vc.dinv.p, I.coef.p + (size_t)(l + 1) * I.coef_stride, vc.b.p, vc.x.p, s);
+    else
+      launch_spmv<T>(view_as<T>(L.R), v.r.p, vc.b.p, s);
   }
   for (int l = nl - 2; l >= 0; --l) {   // upward
     AmgLevel& L = *I.lv[l];
@@ -1448,7 +1612,7 @@ static void vcycle(Amg::Impl& I, const DevSell& Afine) {
     // own rows AND ghost rows of P are applied: the ghost part of x stays consistent with its owner
     // (it was exchanged before the residual), so the first post-smoothing step needs no exchange
     launch_spmv_add<T>(view_as<T>(L.P), vecs<T>(C).x.p, v.x.p, s);
-    smooth<T>(I, L, A, v.b.p, I.opt.postsmooth, false, true);
+    smooth<T>(I, L, A, v.b.p, I.opt.postsmooth, false, true, seams && l == 0 ? kSeamExit : 0);
   }
 }
 
@@ -1456,7 +1620,7 @@ static void vcycle(Amg::Impl& I, const DevSell& Afine) {
 // back after every cycle, so each cycle (and each capture) uses the same buffers in the same roles
 // and a re-capture after a refresh only updates kernel arguments (cudaGraphExecUpdate).
 template <class T>
-static void run_cycle(Amg::Impl& I, const DevSell& Afine) {
+static void run_cycle(Amg::Impl& I, const DevSell& Afine, bool seams = false) {
   cudaStream_t s = I.s;
   std::vector<std::pair<T*, T*>> saved;
   for (auto& L : I.lv) saved.push_back({vecs<T>(*L).x.p, vecs<T>(*L).x2.p});
@@ -1465,17 +1629,21 @@ static void run_cycle(Amg::Impl& I, const DevSell& Afine) {
     for (size_t l = 0; l < I.lv.size(); ++l) { vecs<T>(*I.lv[l]).x.p = saved[l].first; vecs<T>(*I.lv[l]).x2.p = saved[l].second; }
   };
   if (!I.opt.cuda_graph || !I.warm) {
-    vcycle<T>(I, Afine);
+    vcycle<T>(I, Afine, seams);
     restore();
     I.warm = true;
     return;
   }
+  const void* key[5] = {Afine.slice_ptr.p, Afine.col.p, Afine.val.p, Afine.valf.p, Afine.valh.p};
+  if (!std::equal(key, key + 5, I.graph_key) || seams != I.graph_seams) I.graph_valid = false;
   if (!I.graph_valid) {
+    std::copy(key, key + 5, I.graph_key);
+    I.graph_seams = seams;
     const int64_t before = g_kernel_launches;
     SHAKTI_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeRelaxed));
     cudaGraph_t graph = nullptr;
     try {
-      vcycle<T>(I, Afine);
+      vcycle<T>(I, Afine, seams);
     } catch (...) {
       cudaStreamEndCapture(s, &graph);
       if (graph) cudaGraphDestroy(graph);
@@ -1509,8 +1677,8 @@ bool Amg::launch_level_smoother(int level, const DevSell& Afine, int64_t* rows, 
   if (nnz) *nnz = A.nnz;
   if (value_bytes) *value_bytes = uses_half(I, A) ? 2 : (I.opt.fp32_cycle ? 4 : 8);
   if (L.n == 0) return true;
-  if (I.opt.fp32_cycle) cheby_step<float>(I, A, L.vf.dinv.p, L.vf.b.p, L.vf.x.p, L.vf.d.p, L.vf.x2.p, 0.3, 0.2, I.s);
-  else launch_cheby<double>(view(A), L.vd.dinv.p, L.vd.b.p, L.vd.x.p, L.vd.d.p, L.vd.x2.p, 0.3, 0.2, I.s);
+  if (I.opt.fp32_cycle) cheby_step<float>(I, A, L.vf.dinv.p, L.vf.b.p, L.vf.x.p, L.vf.d.p, L.vf.x2.p, I.fixed_coef.p, I.s);
+  else launch_cheby<double>(view(A), L.vd.dinv.p, L.vd.b.p, L.vd.x.p, L.vd.d.p, L.vd.x2.p, I.fixed_coef.p, I.s);
   return true;
 }
 
@@ -1524,11 +1692,32 @@ template double* Amg::rhs_buffer<double>();
 template const float* Amg::cycle<float>(const DevSell&);
 template const double* Amg::cycle<double>(const DevSell&);
 
+// Do the cycle's seams with the Krylov vectors fuse into the fine level's first and last smoothing steps?
+// That takes the mixed-precision cycle with Chebyshev smoothing of the fine level on its fp32 copy, a first
+// step followed by at least one more (the fused start leaves d unwritten) and at least one post-smoothing step.
+static bool seams_apply(const Amg::Impl& I, const DevSell& Afine) {
+  const AmgLevel& L0 = *I.lv[0];
+  return I.opt.fp32_cycle && I.opt.smoother == 1 && I.opt.presmooth >= 2 && I.opt.postsmooth >= 1 && !L0.last &&
+         I.tail_level != 0 && L0.n > 0 && !uses_half(I, Afine);
+}
+
 void Amg::apply(const DevSell& Afine, const double* rin, double* z) {
   Impl& I = *p_;
   cudaStream_t s = I.s;
   AmgLevel& L0 = *I.lv[0];
-  if (I.opt.fp32_cycle) {
+  if (seams_apply(I, Afine)) {
+    // entry and exit read and write the Krylov vectors, which change every iteration: launched outside the graph
+    SHAKTI_LAUNCH(amg_cycle_entry_kernel, div_up(L0.n, 256), 256, 0, s, L0.n, rin, L0.vf.dinv.p, I.coef.p, L0.vf.b.p, L0.vf.x.p);
+    run_cycle<float>(I, Afine, true);
+    const double* cf = I.coef.p + 2 + 2 * (I.opt.postsmooth - 1);
+    const SellViewT<float> A = viewf(Afine);
+    if (A.n_rows < kChebyWideRowsBelow)
+      SHAKTI_LAUNCH((amg_cheby_kernel<float, 8, CHEBY_EXIT>), A.n_slices, 256, 0, s, A, L0.vf.dinv.p, L0.vf.b.p, I.exit_x, L0.vf.d.p,
+                    nullptr, cf, z);
+    else
+      SHAKTI_LAUNCH((amg_cheby_kernel<float, 1, CHEBY_EXIT>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, L0.vf.dinv.p,
+                    L0.vf.b.p, I.exit_x, L0.vf.d.p, nullptr, cf, z);
+  } else if (I.opt.fp32_cycle) {
     launch_d2f(L0.n, rin, L0.vf.b.p, s);
     run_cycle<float>(I, Afine);
     launch_f2d(L0.n, static_cast<const float*>(I.result_ptr), z, s);

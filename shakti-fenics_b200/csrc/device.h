@@ -121,6 +121,9 @@ template <class T> void launch_residual(SellViewT<T> A, const T* x, const T* b, 
 // x_out = x + omega * dinv .* (b - A x)
 template <class T> void launch_jacobi(SellViewT<T> A, const T* dinv, const T* b, const T* x, T* x_out, double omega, cudaStream_t s);
 template <class T> void launch_spmv_add(SellViewT<T> A, const T* x, T* y, cudaStream_t s);             // y += A x
+// b_c = R r and the first Chebyshev step from a zero guess on the coarse level, x_c = dinv_c b_c inv_theta[0]
+template <class T>
+void launch_restrict_cheby_first(SellViewT<T> R, const T* r, const T* dinv_c, const double* inv_theta, T* b_c, T* x_c, cudaStream_t s);
 template <class T> void launch_scaled_mul(int64_t n, const T* a, const T* b, double scale, T* out, cudaStream_t s);  // out = scale a.*b
 template <class T> void launch_fill_t(int64_t n, T v, T* x, cudaStream_t s);
 void launch_d2f(int64_t n, const double* a, float* out, cudaStream_t s);

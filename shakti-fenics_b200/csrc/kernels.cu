@@ -811,6 +811,34 @@ static void spmv_launch(SellViewT<T> A, const T* x, const T* b, const T* dinv, d
   const int64_t threads = (int64_t)A.n_slices * 32;
   SHAKTI_LAUNCH_PDL((spmv_sell_kernel<MODE, T, 1>), div_up(threads, 256), 256, 0, s, A, x, b, dinv, (T)omega, y);
 }
+// Restriction that also takes the coarse level's first Chebyshev step from a zero guess: b_c = R r and
+// x_c = (dinv_c b_c)/theta_c -- spmv_sell_kernel<SPMV_SET> and amg_cheby_first_kernel (amg.cu) in one pass,
+// same operations in the same order.  d is not written; the coarse level's next sweep reads x_c in its place.
+template <class T, int KG>
+__global__ void __launch_bounds__(256)
+restrict_cheby_first_kernel(SellViewT<T> R, const T* __restrict__ r, const T* __restrict__ dinv_c,
+                            const double* __restrict__ inv_theta, T* __restrict__ b_c, T* __restrict__ x_c) {
+  pdl_sync();
+  int32_t row;
+  T acc;
+  if (!sell_row_dot<T, KG>(R, r, row, acc)) return;
+  b_c[row] = acc;
+  x_c[row] = dinv_c[row] * acc * (T)inv_theta[0];
+}
+template <class T>
+void launch_restrict_cheby_first(SellViewT<T> R, const T* r, const T* dinv_c, const double* inv_theta, T* b_c, T* x_c, cudaStream_t s) {
+  if (R.n_rows == 0) return;
+  if (R.n_rows < kWideRowsBelow)
+    SHAKTI_LAUNCH_PDL((restrict_cheby_first_kernel<T, 8>), R.n_slices, 256, 0, s, R, r, dinv_c, inv_theta, b_c, x_c);
+  else
+    SHAKTI_LAUNCH_PDL((restrict_cheby_first_kernel<T, 1>), div_up((int64_t)R.n_slices * 32, 256), 256, 0, s, R, r, dinv_c, inv_theta,
+                      b_c, x_c);
+}
+template void launch_restrict_cheby_first<double>(SellViewT<double>, const double*, const double*, const double*, double*, double*,
+                                                  cudaStream_t);
+template void launch_restrict_cheby_first<float>(SellViewT<float>, const float*, const float*, const double*, float*, float*,
+                                                 cudaStream_t);
+
 template <class T> void launch_spmv(SellViewT<T> A, const T* x, T* y, cudaStream_t s) { spmv_launch<SPMV_SET, T>(A, x, nullptr, nullptr, 0, y, s); }
 template <class T> void launch_spmv_add(SellViewT<T> A, const T* x, T* y, cudaStream_t s) { spmv_launch<SPMV_ADD, T>(A, x, nullptr, nullptr, 0, y, s); }
 template <class T> void launch_residual(SellViewT<T> A, const T* x, const T* b, T* r, cudaStream_t s) { spmv_launch<SPMV_RESID, T>(A, x, b, nullptr, 0, r, s); }
