@@ -320,6 +320,13 @@ int shakti_time_kernel(shakti_model* m, int which, int reps, double dt, double* 
  * (value_bytes + 4) * nnz + 7 * vector_bytes * rows.  Needs a built hierarchy (run a step). */
 int shakti_time_amg_smoother(shakti_model* m, int level, int reps, double* ms_per_launch, int64_t* rows,
                              int64_t* nnz, int32_t* value_bytes, int32_t* vector_bytes);
+/* One launch of a SELL kernel of AMG level `level`'s part of the V-cycle, launched as the cycle launches it and
+ * timed the same way.  `which`: 0 = smoothing step (as shakti_time_amg_smoother), 1 = residual r = b - A x,
+ * 2 = restriction onto level + 1 (with that level's first Chebyshev step where the cycle fuses the two),
+ * 3 = prolongation x += P x_coarse.  info = {rows, columns, stored entries, longest row, bytes per stored value}
+ * of the kernel's matrix (A, R or P), then bytes per vector entry and 1 if the restriction is the fused one.
+ * SHAKTI_ERR_INVALID for a kernel the cycle does not run on this rank. */
+int shakti_time_amg_level_kernel(shakti_model* m, int level, int which, int reps, double* ms_per_launch, int64_t info[7]);
 /* Algorithmic bytes per launch of kernel `which` (SURVEY.md §8d formulas). */
 int shakti_kernel_bytes(shakti_model* m, int which, double* bytes);
 

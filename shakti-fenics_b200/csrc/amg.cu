@@ -405,12 +405,13 @@ __global__ void amg_dense_apply_kernel(int32_t n, const double* __restrict__ D, 
 // ------------------------------------------------------------------ smoother kernels
 // Chebyshev step: r = dinv (b - A x); d = c1 d + c2 r; x_out = x + d
 // KG as in spmv_sell_kernel (kernels.cu): 1 = thread per row, 8 = block per slice for small wide-rowed levels.
+// RB (KG = 1): row bound of sell_row_product (sell_row.h), picked by sell_row_bound_dispatch from the longest row.
 // cf = {c1, c2} in device memory (amg_cheby_coef_kernel), so that a new spectral bound changes no kernel argument.
 // MODE, for the fine level of the mixed-precision cycle (Amg::apply):
 //   CHEBY_X_IS_D  first sweep after amg_cycle_entry_kernel, which wrote the first iterate to x only: the old d is x
 //   CHEBY_EXIT    last sweep of the cycle: z = (double)(x + d_new); d is read, d and x_out are not written
 enum { CHEBY_PLAIN = 0, CHEBY_X_IS_D = 1, CHEBY_EXIT = 2 };
-template <class T, int KG, int MODE = CHEBY_PLAIN>
+template <class T, int KG, int MODE = CHEBY_PLAIN, int RB = 0>
 __global__ void __launch_bounds__(256)
 amg_cheby_kernel(SellViewT<T> A, const T* __restrict__ dinv, const T* __restrict__ b, const T* __restrict__ x,
                  T* __restrict__ d, T* __restrict__ x_out, const double* __restrict__ cf, double* __restrict__ z) {
@@ -423,10 +424,7 @@ amg_cheby_kernel(SellViewT<T> A, const T* __restrict__ dinv, const T* __restrict
     if (slice >= A.n_slices) return;
     const int32_t base = A.slice_ptr[slice];
     const int32_t w = (A.slice_ptr[slice + 1] - base) >> 5;
-    const int32_t* __restrict__ cp = A.col + base + (row & 31);
-    const T* __restrict__ vp = A.val + base + (row & 31);
-#pragma unroll 4
-    for (int k = 0; k < w; ++k) acc += vp[32 * k] * x[cp[32 * k]];
+    acc = sell_row_product<RB>(A.col + base + (row & 31), A.val + base + (row & 31), w, x);
   } else {
     __shared__ T psum[KG][32];
     const int32_t slice = blockIdx.x;
@@ -462,8 +460,10 @@ static void launch_cheby(SellViewT<T> A, const T* dinv, const T* b, const T* x, 
   if (A.n_rows < kChebyWideRowsBelow)
     SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 8, MODE>), A.n_slices, 256, 0, s, A, dinv, b, x, d, x_out, cf, nullptr);
   else
-    SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 1, MODE>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, dinv, b, x, d, x_out, cf,
-                      nullptr);
+    sell_row_bound_dispatch<T>(A.max_width, [&](auto rb) {
+      SHAKTI_LAUNCH_PDL((amg_cheby_kernel<T, 1, MODE, rb.value>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, dinv, b, x, d,
+                        x_out, cf, nullptr);
+    });
 }
 
 // ---- the same two kernels of the LARGE levels on the half-precision, row-scaled copy Ah = D^-1 A (unit
@@ -481,11 +481,7 @@ amg_cheby_h_kernel(int32_t n_rows, int32_t n_slices, const int32_t* __restrict__
   if (slice >= n_slices) return;
   const int32_t base = slice_ptr[slice];
   const int32_t w = (slice_ptr[slice + 1] - base) >> 5;
-  const int32_t* __restrict__ cp = col + base + (row & 31);
-  const __half* __restrict__ vp = val + base + (row & 31);
-  float acc = 0.f;
-#pragma unroll 4
-  for (int k = 0; k < w; ++k) acc += __half2float(vp[32 * k]) * x[cp[32 * k]];
+  const float acc = sell_row_product<0>(col + base + (row & 31), val + base + (row & 31), w, x);
   if (row >= n_rows) return;
   const float c1 = (float)cf[0], c2 = (float)cf[1];
   const float r = dinv[row] * b[row] - acc;
@@ -504,11 +500,7 @@ amg_resid_h_kernel(int32_t n_rows, int32_t n_slices, const int32_t* __restrict__
   if (slice >= n_slices) return;
   const int32_t base = slice_ptr[slice];
   const int32_t w = (slice_ptr[slice + 1] - base) >> 5;
-  const int32_t* __restrict__ cp = col + base + (row & 31);
-  const __half* __restrict__ vp = val + base + (row & 31);
-  float acc = 0.f;
-#pragma unroll 4
-  for (int k = 0; k < w; ++k) acc += __half2float(vp[32 * k]) * x[cp[32 * k]];
+  const float acc = sell_row_product<0>(col + base + (row & 31), val + base + (row & 31), w, x);
   if (row >= n_rows) return;
   const float di = dinv[row];
   r[row] = b[row] - (di != 0.f ? acc / di : 0.f);
@@ -1682,6 +1674,38 @@ bool Amg::launch_level_smoother(int level, const DevSell& Afine, int64_t* rows, 
   return true;
 }
 
+template <class T>
+static void level_kernel(Amg::Impl& I, int l, int which, const DevSell& A) {
+  AmgLevel& L = *I.lv[l];
+  CycleVecs<T>& v = vecs<T>(L);
+  CycleVecs<T>& vc = vecs<T>(*I.lv[l + (which == 1 ? 0 : 1)]);
+  if (which == 1) level_residual<T>(I, A, v.dinv.p, v.x.p, v.b.p, v.r.p, I.s);
+  else if (which == 3) launch_spmv_add<T>(view_as<T>(L.P), vc.x.p, v.x.p, I.s);
+  else if (restrict_starts(I, l + 1))
+    launch_restrict_cheby_first<T>(view_as<T>(L.R), v.r.p, vc.dinv.p, I.coef.p + (size_t)(l + 1) * I.coef_stride, vc.b.p, vc.x.p, I.s);
+  else
+    launch_spmv<T>(view_as<T>(L.R), v.r.p, vc.b.p, I.s);
+}
+bool Amg::launch_level_kernel(int level, int which, const DevSell& Afine, int64_t info[7]) {
+  Impl& I = *p_;
+  if (!I.built || level < 0 || level >= (int)I.lv.size() || which < 0 || which > 3) return false;
+  AmgLevel& L = *I.lv[level];
+  const DevSell& A = (level == 0) ? Afine : L.A;
+  // the cycle restricts and prolongs only between levels it runs on this rank
+  const bool transfer = !L.last && level + 1 < (int)I.lv.size() && (I.tail_level < 0 || level < I.tail_level);
+  if (which >= 2 && !transfer) return false;
+  const DevSell& M = which == 2 ? L.R : which == 3 ? L.P : A;
+  info[0] = M.n_rows; info[1] = M.n_cols; info[2] = M.nnz; info[3] = M.max_width;
+  info[4] = &M == &A && uses_half(I, A) ? 2 : (I.opt.fp32_cycle ? 4 : 8);   // R and P have no half-precision copy
+  info[5] = I.opt.fp32_cycle ? 4 : 8;
+  info[6] = which == 2 && restrict_starts(I, level + 1);
+  if (which == 0) return launch_level_smoother(level, Afine, nullptr, nullptr);
+  if (M.n_rows == 0) return true;
+  if (I.opt.fp32_cycle) level_kernel<float>(I, level, which, A);
+  else level_kernel<double>(I, level, which, A);
+  return true;
+}
+
 template <class T> T* Amg::rhs_buffer() { return vecs<T>(*p_->lv[0]).b.p; }
 template <class T> const T* Amg::cycle(const DevSell& Afine) {
   run_cycle<T>(*p_, Afine);
@@ -1715,8 +1739,10 @@ void Amg::apply(const DevSell& Afine, const double* rin, double* z) {
       SHAKTI_LAUNCH((amg_cheby_kernel<float, 8, CHEBY_EXIT>), A.n_slices, 256, 0, s, A, L0.vf.dinv.p, L0.vf.b.p, I.exit_x, L0.vf.d.p,
                     nullptr, cf, z);
     else
-      SHAKTI_LAUNCH((amg_cheby_kernel<float, 1, CHEBY_EXIT>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, L0.vf.dinv.p,
-                    L0.vf.b.p, I.exit_x, L0.vf.d.p, nullptr, cf, z);
+      sell_row_bound_dispatch<float>(A.max_width, [&](auto rb) {
+        SHAKTI_LAUNCH((amg_cheby_kernel<float, 1, CHEBY_EXIT, rb.value>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A,
+                      L0.vf.dinv.p, L0.vf.b.p, I.exit_x, L0.vf.d.p, nullptr, cf, z);
+      });
   } else if (I.opt.fp32_cycle) {
     launch_d2f(L0.n, rin, L0.vf.b.p, s);
     run_cycle<float>(I, Afine);

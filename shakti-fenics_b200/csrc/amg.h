@@ -60,6 +60,11 @@ class Amg {
   // micro-benchmark hook: one smoothing step (SpMV fused with the Chebyshev recurrence) of level `level` on
   // the cycle's own vectors; rows / stored entries of that level's operator are returned for the roofline
   bool launch_level_smoother(int level, const DevSell& Afine, int64_t* rows, int64_t* nnz, int* value_bytes = nullptr);
+  // the same for level `level`'s other SELL kernels, launched as the cycle launches them: which = 1 residual,
+  // 2 restriction onto level + 1, 3 prolongation from level + 1 (0: the smoothing step).  info = {rows, columns,
+  // stored entries, longest row, bytes per value of the matrix, bytes per vector entry, 1 if the restriction
+  // also takes the coarse level's first Chebyshev step}.  false: no such kernel on this rank.
+  bool launch_level_kernel(int level, int which, const DevSell& Afine, int64_t info[7]);
   int levels() const;
   double operator_complexity() const;
   int64_t refreshes() const { return refreshes_; }

@@ -1477,6 +1477,27 @@ int shakti_time_amg_smoother(shakti_model* m, int level, int reps, double* ms_pe
   SHAKTI_CATCH
 }
 
+int shakti_time_amg_level_kernel(shakti_model* m, int level, int which, int reps, double* ms_per_launch, int64_t info[7]) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && ms_per_launch && info && reps > 0, "bad arguments");
+  use_device(m);
+  SHAKTI_REQUIRE(m->amg && m->amg->ready() && m->J_valid, "no AMG hierarchy yet: run a step first");
+  SHAKTI_REQUIRE(m->amg->launch_level_kernel(level, which, m->J, info), "no such AMG level kernel on this rank");
+  cudaEvent_t e0, e1;
+  SHAKTI_CUDA(cudaEventCreate(&e0));
+  SHAKTI_CUDA(cudaEventCreate(&e1));
+  SHAKTI_CUDA(cudaEventRecord(e0, m->stream));
+  for (int i = 0; i < reps; ++i) m->amg->launch_level_kernel(level, which, m->J, info);
+  SHAKTI_CUDA(cudaEventRecord(e1, m->stream));
+  SHAKTI_CUDA(cudaEventSynchronize(e1));
+  float ms = 0;
+  SHAKTI_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  *ms_per_launch = (double)ms / reps;
+  SHAKTI_CATCH
+}
+
 int shakti_comm_unique_id(uint8_t id[128]) {
   SHAKTI_TRY
   comm_unique_id(id);

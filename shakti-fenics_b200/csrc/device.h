@@ -4,6 +4,7 @@
 
 #include "common.h"
 #include "prep.h"
+#include "sell_row.h"
 
 namespace shakti {
 
@@ -40,10 +41,11 @@ struct SellViewT {
   const int32_t* slice_ptr;
   const int32_t* col;
   const T* val;
+  int32_t max_width;   // longest row: picks the row bound of the one-thread-per-row kernels (sell_row.h)
 };
 using SellView = SellViewT<double>;
-inline SellView view(const DevSell& a) { return {a.n_rows, a.n_slices, a.slice_ptr.p, a.col.p, a.val.p}; }
-inline SellViewT<float> viewf(const DevSell& a) { return {a.n_rows, a.n_slices, a.slice_ptr.p, a.col.p, a.valf.p}; }
+inline SellView view(const DevSell& a) { return {a.n_rows, a.n_slices, a.slice_ptr.p, a.col.p, a.val.p, a.max_width}; }
+inline SellViewT<float> viewf(const DevSell& a) { return {a.n_rows, a.n_slices, a.slice_ptr.p, a.col.p, a.valf.p, a.max_width}; }
 template <class T> inline SellViewT<T> view_as(const DevSell& a);
 template <> inline SellViewT<double> view_as<double>(const DevSell& a) { return view(a); }
 template <> inline SellViewT<float> view_as<float>(const DevSell& a) { return viewf(a); }

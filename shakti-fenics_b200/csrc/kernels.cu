@@ -750,8 +750,9 @@ enum { SPMV_SET = 0, SPMV_ADD = 1, SPMV_RESID = 2, SPMV_JACOBI = 3 };
 // the 32 rows of a slice).  KG = 8: one 256-thread block per slice, warp g takes the entries k = g, g+8, ...
 // of all 32 rows (still coalesced) and the eight partial sums meet in shared memory.  That is for the small,
 // wide-rowed coarse levels of the AMG hierarchy, where one thread per row is a chain of ~100 dependent
-// gathers (15 us for a 500-row level) and the eight-way split cuts the chain eightfold.
-template <class T, int KG>
+// gathers (15 us for a 500-row level) and the eight-way split cuts the chain eightfold.  RB: row bound of the
+// KG = 1 row product (sell_row.h), which amg.cu's one-thread-per-row kernels share.
+template <class T, int KG, int RB>
 __device__ __forceinline__ bool sell_row_dot(const SellViewT<T>& A, const T* __restrict__ x, int32_t& row, T& acc) {
   if (KG == 1) {
     row = blockIdx.x * blockDim.x + threadIdx.x;
@@ -759,11 +760,7 @@ __device__ __forceinline__ bool sell_row_dot(const SellViewT<T>& A, const T* __r
     if (slice >= A.n_slices) return false;
     const int32_t base = A.slice_ptr[slice];
     const int32_t w = (A.slice_ptr[slice + 1] - base) >> 5;
-    const int32_t* __restrict__ cp = A.col + base + (row & 31);
-    const T* __restrict__ vp = A.val + base + (row & 31);
-    acc = 0;
-#pragma unroll 4
-    for (int k = 0; k < w; ++k) acc += vp[32 * k] * x[cp[32 * k]];
+    acc = sell_row_product<RB>(A.col + base + (row & 31), A.val + base + (row & 31), w, x);
     return row < A.n_rows;
   } else {
     __shared__ T psum[KG][32];
@@ -787,14 +784,14 @@ __device__ __forceinline__ bool sell_row_dot(const SellViewT<T>& A, const T* __r
 }
 constexpr int32_t kWideRowsBelow = 300000;   // matrices with fewer rows use the KG = 8 kernels
 
-template <int MODE, class T, int KG>
+template <int MODE, class T, int KG, int RB = 0>
 __global__ void __launch_bounds__(256)
 spmv_sell_kernel(SellViewT<T> A, const T* __restrict__ x, const T* __restrict__ b, const T* __restrict__ dinv, T omega,
                  T* __restrict__ y) {
   pdl_sync();
   int32_t row;
   T acc;
-  if (!sell_row_dot<T, KG>(A, x, row, acc)) return;
+  if (!sell_row_dot<T, KG, RB>(A, x, row, acc)) return;
   if (MODE == SPMV_SET) y[row] = acc;
   else if (MODE == SPMV_ADD) y[row] += acc;
   else if (MODE == SPMV_RESID) y[row] = b[row] - acc;
@@ -808,20 +805,21 @@ static void spmv_launch(SellViewT<T> A, const T* x, const T* b, const T* dinv, d
     SHAKTI_LAUNCH_PDL((spmv_sell_kernel<MODE, T, 8>), A.n_slices, 256, 0, s, A, x, b, dinv, (T)omega, y);
     return;
   }
-  const int64_t threads = (int64_t)A.n_slices * 32;
-  SHAKTI_LAUNCH_PDL((spmv_sell_kernel<MODE, T, 1>), div_up(threads, 256), 256, 0, s, A, x, b, dinv, (T)omega, y);
+  sell_row_bound_dispatch<T>(A.max_width, [&](auto rb) {
+    SHAKTI_LAUNCH_PDL((spmv_sell_kernel<MODE, T, 1, rb.value>), div_up((int64_t)A.n_slices * 32, 256), 256, 0, s, A, x, b, dinv, (T)omega, y);
+  });
 }
 // Restriction that also takes the coarse level's first Chebyshev step from a zero guess: b_c = R r and
 // x_c = (dinv_c b_c)/theta_c -- spmv_sell_kernel<SPMV_SET> and amg_cheby_first_kernel (amg.cu) in one pass,
 // same operations in the same order.  d is not written; the coarse level's next sweep reads x_c in its place.
-template <class T, int KG>
+template <class T, int KG, int RB = 0>
 __global__ void __launch_bounds__(256)
 restrict_cheby_first_kernel(SellViewT<T> R, const T* __restrict__ r, const T* __restrict__ dinv_c,
                             const double* __restrict__ inv_theta, T* __restrict__ b_c, T* __restrict__ x_c) {
   pdl_sync();
   int32_t row;
   T acc;
-  if (!sell_row_dot<T, KG>(R, r, row, acc)) return;
+  if (!sell_row_dot<T, KG, RB>(R, r, row, acc)) return;
   b_c[row] = acc;
   x_c[row] = dinv_c[row] * acc * (T)inv_theta[0];
 }
@@ -831,8 +829,10 @@ void launch_restrict_cheby_first(SellViewT<T> R, const T* r, const T* dinv_c, co
   if (R.n_rows < kWideRowsBelow)
     SHAKTI_LAUNCH_PDL((restrict_cheby_first_kernel<T, 8>), R.n_slices, 256, 0, s, R, r, dinv_c, inv_theta, b_c, x_c);
   else
-    SHAKTI_LAUNCH_PDL((restrict_cheby_first_kernel<T, 1>), div_up((int64_t)R.n_slices * 32, 256), 256, 0, s, R, r, dinv_c, inv_theta,
-                      b_c, x_c);
+    sell_row_bound_dispatch<T>(R.max_width, [&](auto rb) {
+      SHAKTI_LAUNCH_PDL((restrict_cheby_first_kernel<T, 1, rb.value>), div_up((int64_t)R.n_slices * 32, 256), 256, 0, s, R, r, dinv_c,
+                        inv_theta, b_c, x_c);
+    });
 }
 template void launch_restrict_cheby_first<double>(SellViewT<double>, const double*, const double*, const double*, double*, double*,
                                                   cudaStream_t);

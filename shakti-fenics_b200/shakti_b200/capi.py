@@ -514,6 +514,19 @@ class Model:
         by = (vb.value + 4) * nnz.value + 7 * xb.value * rows.value
         return dict(ms=ms.value, rows=rows.value, nnz=nnz.value, value_bytes=vb.value, vector_bytes=xb.value, bytes=by)
 
+    AMG_LEVEL_KERNELS = {"smoother": 0, "residual": 1, "restriction": 2, "prolongation": 3}
+
+    def time_amg_level_kernel(self, level, which, reps=20):
+        """-> dict(ms, rows, cols, nnz, max_width, value_bytes, vector_bytes, fused) for one launch of SELL kernel
+        `which` (AMG_LEVEL_KERNELS) of AMG level `level`, launched as the V-cycle launches it; the shape and value
+        bytes are those of the kernel's matrix (A, R or P); fused: the restriction takes the coarse level's first
+        Chebyshev step too."""
+        ms, info = C.c_double(0), (C.c_int64 * 7)()
+        _check(self.lib.shakti_time_amg_level_kernel(self._h, C.c_int(level), C.c_int(self.AMG_LEVEL_KERNELS[which]),
+                                                     C.c_int(reps), C.byref(ms), info))
+        return dict(ms=ms.value, rows=info[0], cols=info[1], nnz=info[2], max_width=info[3], value_bytes=info[4],
+                    vector_bytes=info[5], fused=bool(info[6]))
+
     def kernel_bytes(self, which):
         b = C.c_double(0)
         _check(self.lib.shakti_kernel_bytes(self._h, C.c_int(self.KERNELS[which]), C.byref(b)))
