@@ -330,6 +330,32 @@ int shakti_time_amg_level_kernel(shakti_model* m, int level, int which, int reps
 /* Algorithmic bytes per launch of kernel `which` (SURVEY.md §8d formulas). */
 int shakti_kernel_bytes(shakti_model* m, int which, double* bytes);
 
+/* ---------------------------------------------------------------- AMG test hooks
+ * What the preconditioner computes, level by level, for a comparison with a float64 reference (tests/amg_reference.py).
+ * One rank only (SHAKTI_ERR_INVALID on several); rows and columns are in the model's internal order, which
+ * shakti_get_owned maps to caller ids.  They add no work to the solver's own calls.
+ * shakti_amg_refresh: rebuilds the preconditioner from the last assembled Jacobian -- full = 1: the whole hierarchy's
+ *   numbers (the first call also builds the hierarchy); full = 0: only the fine smoother (diagonal and Chebyshev
+ *   bound), the rest stays lagged, as a Newton solve between two scheduled refreshes does.
+ * shakti_amg_level_info: info[18] = {rows, columns, n_coarse (0 on the last level), stored entries and longest row of
+ *   A, of P, of R (0 on the last level), last, dense coarsest solve (last level only), A runs on its half-precision
+ *   copy, the restriction onto this level takes its first Chebyshev step, the cycle's first and last fine sweeps
+ *   are fused with its entry and exit (same on every level), number of levels, fp32 cycle, AP and RAP of this level
+ *   ran the table-driven SpGEMM}.
+ * shakti_amg_get_matrix: `which` 0 = A (level 0: the fine Jacobian), 1 = P, 2 = R, 3 = the fp32 copy of A the cycle
+ *   reads, 4 = the fp16 copy of D^-1 A; as CSR (sorted columns), values widened to double.  Call with NULL arrays to
+ *   query nnz (rowptr holds rows + 1 entries).
+ * shakti_amg_get_vectors: level's dinv (rows doubles) in fp64 and in the cycle's precision, its Chebyshev bound of
+ *   lambda_max(D^-1 A) and coefficient table ({1/theta, -, then (c1, c2) of sweep k at 2 + 2k}, *stride doubles;
+ *   stride 0 without the Chebyshev smoother).  Any pointer may be NULL.
+ * shakti_amg_apply: z = M^-1 r (n_owned doubles each), one V-cycle through the path a Krylov iteration takes. */
+int shakti_amg_refresh(shakti_model* m, int full);
+int shakti_amg_level_info(shakti_model* m, int level, int64_t info[18]);
+int shakti_amg_get_matrix(shakti_model* m, int level, int which, int32_t* rowptr, int32_t* col, double* val, int64_t* nnz);
+int shakti_amg_get_vectors(shakti_model* m, int level, double* dinv, double* dinv_cycle, double* lmax, double* coef,
+                           int32_t* stride);
+int shakti_amg_apply(shakti_model* m, const double* r, double* z);
+
 /* ---------------------------------------------------------------- multi-GPU
  * One process per GPU.  Rank 0 calls shakti_comm_unique_id, the 128-byte id is broadcast by
  * the host program (torch.distributed), then every rank calls shakti_comm_init BEFORE

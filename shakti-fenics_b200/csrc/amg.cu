@@ -1754,6 +1754,90 @@ void Amg::apply(const DevSell& Afine, const double* rin, double* z) {
   }
 }
 
+// ------------------------------------------------------------------ test hooks (one rank)
+bool Amg::level_info(int level, const DevSell& Afine, int64_t info[18]) const {
+  const Impl& I = *p_;
+  if (!I.built || level < 0 || level >= (int)I.lv.size()) return false;
+  const AmgLevel& L = *I.lv[level];
+  const DevSell& A = (level == 0) ? Afine : L.A;
+  info[0] = L.n; info[1] = L.n_cols; info[2] = L.last ? 0 : L.n_coarse;
+  info[3] = A.nnz; info[4] = A.max_width;
+  info[5] = L.last ? 0 : L.P.nnz; info[6] = L.last ? 0 : L.P.max_width;
+  info[7] = L.last ? 0 : L.R.nnz; info[8] = L.last ? 0 : L.R.max_width;
+  info[9] = L.last;
+  info[10] = L.last && I.dense_coarse;
+  info[11] = uses_half(I, A);
+  info[12] = level > 0 && restrict_starts(I, level);
+  info[13] = seams_apply(I, Afine);
+  info[14] = (int64_t)I.lv.size();
+  info[15] = I.opt.fp32_cycle != 0;
+  // the numeric products of this level ran the table-driven kernel (spgemm_numeric)
+  info[16] = !L.last && L.n > 400000 && L.plan_AP.ok;
+  info[17] = !L.last && L.n_coarse > 400000 && L.plan_RAP.ok;
+  return true;
+}
+
+bool Amg::level_matrix(int level, int which, const DevSell& Afine, HostCsr& csr, std::vector<double>& val) const {
+  const Impl& I = *p_;
+  if (!I.built || level < 0 || level >= (int)I.lv.size() || which < 0 || which > 4) return false;
+  const AmgLevel& L = *I.lv[level];
+  const DevSell& A = (level == 0) ? Afine : L.A;
+  if ((which == 1 || which == 2) && L.last) return false;
+  const DevSell& M = which == 1 ? L.P : which == 2 ? L.R : A;
+  std::vector<double> v;
+  if (which == 3) {
+    if (M.valf.n != (size_t)M.padded) return false;
+    for (float f : M.valf.download(I.s)) v.push_back((double)f);
+  } else if (which == 4) {
+    if (M.valh.n < (size_t)M.padded || M.padded == 0) return false;
+    const std::vector<__half> h = M.valh.download(I.s);
+    for (int64_t k = 0; k < M.padded; ++k) v.push_back((double)__half2float(h[k]));
+  } else {
+    v = M.val.download(I.s);
+  }
+  const std::vector<int32_t> sp = M.slice_ptr.download(I.s), col = M.col.download(I.s), len = M.rowlen.download(I.s);
+  csr = HostCsr();
+  csr.n_rows = M.n_rows;
+  csr.n_cols = M.n_cols;
+  csr.rowptr.assign((size_t)M.n_rows + 1, 0);
+  val.clear();
+  for (int32_t r = 0; r < M.n_rows; ++r) {
+    for (int32_t k = 0; k < len[r]; ++k) {
+      const int64_t p = (int64_t)sp[r >> 5] + 32 * (int64_t)k + (r & 31);
+      csr.col.push_back(col[p]);
+      val.push_back(v[p]);
+    }
+    csr.rowptr[r + 1] = (int32_t)csr.col.size();
+  }
+  return true;
+}
+
+bool Amg::level_vectors(int level, std::vector<double>& dinv, std::vector<double>& dinv_cycle, double& lmax,
+                        std::vector<double>& coef, int& stride) const {
+  const Impl& I = *p_;
+  if (!I.built || level < 0 || level >= (int)I.lv.size()) return false;
+  const AmgLevel& L = *I.lv[level];
+  dinv = L.dinv.download(I.s);
+  dinv.resize(L.n);
+  if (I.opt.fp32_cycle) {
+    dinv_cycle.clear();
+    for (float f : L.vf.dinv.download(I.s)) dinv_cycle.push_back((double)f);
+  } else {
+    dinv_cycle = L.vd.dinv.download(I.s);
+  }
+  dinv_cycle.resize(L.n);
+  lmax = 0.0;
+  coef.clear();
+  stride = 0;
+  if (I.opt.smoother == 1 && I.lmax.n > (size_t)level) {
+    lmax = I.lmax.download(I.s)[level];
+    stride = I.coef_stride;
+    const std::vector<double> c = I.coef.download(I.s);
+    coef.assign(c.begin() + (size_t)level * stride, c.begin() + (size_t)(level + 1) * stride);
+  }
+  return true;
+}
+
 }  // namespace shakti
 
 // ---------------------------------------------------------------- host-only test hook

@@ -65,6 +65,16 @@ class Amg {
   // stored entries, longest row, bytes per value of the matrix, bytes per vector entry, 1 if the restriction
   // also takes the coarse level's first Chebyshev step}.  false: no such kernel on this rank.
   bool launch_level_kernel(int level, int which, const DevSell& Afine, int64_t info[7]);
+  // ---- test hooks (one rank; the shakti_amg_* functions of the C ABI).  false: no such level / matrix.
+  // info: the layout of shakti_amg_level_info (shakti_b200.h)
+  bool level_info(int level, const DevSell& Afine, int64_t info[18]) const;
+  // matrix `which` of level `level` (0 A, 1 P, 2 R, 3 the fp32 copy of A, 4 the fp16 copy of D^-1 A) as a CSR in the
+  // level's numbering, values widened to double
+  bool level_matrix(int level, int which, const DevSell& Afine, HostCsr& csr, std::vector<double>& val) const;
+  // the level's smoother diagonal in fp64 and in the cycle's precision, its Chebyshev bound and coefficients
+  // (amg_cheby_coef_kernel: stride doubles; empty without the Chebyshev smoother)
+  bool level_vectors(int level, std::vector<double>& dinv, std::vector<double>& dinv_cycle, double& lmax,
+                     std::vector<double>& coef, int& stride) const;
   int levels() const;
   double operator_complexity() const;
   int64_t refreshes() const { return refreshes_; }

@@ -1498,6 +1498,81 @@ int shakti_time_amg_level_kernel(shakti_model* m, int level, int which, int reps
   SHAKTI_CATCH
 }
 
+// ---- AMG test hooks: one rank, where internal numbering = the rank's owned order
+static void require_amg_hook(shakti_model* m, bool need_hierarchy) {
+  SHAKTI_REQUIRE(m, "null model");
+  SHAKTI_REQUIRE(!comm().active(), "the AMG test hooks run on one rank only");
+  use_device(m);
+  SHAKTI_REQUIRE(m->J_valid, "no assembled Jacobian");
+  if (need_hierarchy) SHAKTI_REQUIRE(m->amg && m->amg->ready(), "no AMG hierarchy yet: call shakti_amg_refresh first");
+}
+
+int shakti_amg_refresh(shakti_model* m, int full) {
+  SHAKTI_TRY
+  require_amg_hook(m, false);
+  ensure_amg(m);
+  if (full) {
+    m->amg->refresh(m->J, m->diag_pos.p);
+    m->st.amg_refreshes++;
+  } else {
+    SHAKTI_REQUIRE(m->amg->ready(), "no AMG hierarchy to keep: refresh it in full first");
+    m->amg->refresh_fine_smoother(m->J, m->diag_pos.p);
+  }
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
+  SHAKTI_CATCH
+}
+
+int shakti_amg_level_info(shakti_model* m, int level, int64_t info[18]) {
+  SHAKTI_TRY
+  require_amg_hook(m, true);
+  SHAKTI_REQUIRE(info, "null argument");
+  SHAKTI_REQUIRE(m->amg->level_info(level, m->J, info), "no such AMG level");
+  SHAKTI_CATCH
+}
+
+int shakti_amg_get_matrix(shakti_model* m, int level, int which, int32_t* rowptr, int32_t* col, double* val, int64_t* nnz) {
+  SHAKTI_TRY
+  require_amg_hook(m, true);
+  SHAKTI_REQUIRE(nnz, "null argument");
+  HostCsr a;
+  std::vector<double> v;
+  SHAKTI_REQUIRE(m->amg->level_matrix(level, which, m->J, a, v), "no such AMG level matrix");
+  *nnz = a.nnz();
+  if (rowptr) std::copy(a.rowptr.begin(), a.rowptr.end(), rowptr);
+  if (col) std::copy(a.col.begin(), a.col.end(), col);
+  if (val) std::copy(v.begin(), v.end(), val);
+  SHAKTI_CATCH
+}
+
+int shakti_amg_get_vectors(shakti_model* m, int level, double* dinv, double* dinv_cycle, double* lmax, double* coef,
+                           int32_t* stride) {
+  SHAKTI_TRY
+  require_amg_hook(m, true);
+  std::vector<double> d, dc, c;
+  double lm = 0.0;
+  int st = 0;
+  SHAKTI_REQUIRE(m->amg->level_vectors(level, d, dc, lm, c, st), "no such AMG level");
+  if (dinv) std::copy(d.begin(), d.end(), dinv);
+  if (dinv_cycle) std::copy(dc.begin(), dc.end(), dinv_cycle);
+  if (lmax) *lmax = lm;
+  if (coef) std::copy(c.begin(), c.end(), coef);
+  if (stride) *stride = st;
+  SHAKTI_CATCH
+}
+
+int shakti_amg_apply(shakti_model* m, const double* r, double* z) {
+  SHAKTI_TRY
+  require_amg_hook(m, true);
+  SHAKTI_REQUIRE(r && z, "null argument");
+  const int32_t no = m->hm.n_owned;
+  SHAKTI_CUDA(cudaMemcpyAsync(m->rhs.p, r, sizeof(double) * no, cudaMemcpyHostToDevice, m->stream));
+  SHAKTI_CUDA(cudaMemsetAsync(m->dx.p, 0, sizeof(double) * m->hm.n_local, m->stream));
+  m->amg->apply(m->J, m->rhs.p, m->dx.p);
+  SHAKTI_CUDA(cudaMemcpyAsync(z, m->dx.p, sizeof(double) * no, cudaMemcpyDeviceToHost, m->stream));
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
+  SHAKTI_CATCH
+}
+
 int shakti_comm_unique_id(uint8_t id[128]) {
   SHAKTI_TRY
   comm_unique_id(id);

@@ -531,3 +531,55 @@ class Model:
         b = C.c_double(0)
         _check(self.lib.shakti_kernel_bytes(self._h, C.c_int(self.KERNELS[which]), C.byref(b)))
         return b.value
+
+    # ---- AMG test hooks (one rank; internal order: owned() gives the caller id of each row)
+    AMG_INFO = ("rows", "cols", "n_coarse", "A_nnz", "A_width", "P_nnz", "P_width", "R_nnz", "R_width", "last",
+                "dense_coarse", "uses_half", "restrict_starts", "seams_apply", "levels", "fp32_cycle", "table_AP",
+                "table_RAP")
+    AMG_MATRICES = dict(A=0, P=1, R=2, valf=3, valh=4)
+
+    def amg_refresh(self, full=True):
+        """Rebuild the AMG preconditioner from the last assembled Jacobian: the whole hierarchy (full) or only the
+        fine smoother, the rest lagged."""
+        _check(self.lib.shakti_amg_refresh(self._h, C.c_int(1 if full else 0)))
+
+    def amg_level_info(self, level):
+        info = (C.c_int64 * len(self.AMG_INFO))()
+        _check(self.lib.shakti_amg_level_info(self._h, C.c_int(level), info))
+        return dict(zip(self.AMG_INFO, (int(v) for v in info)))
+
+    def amg_matrix(self, level, which):
+        """Matrix `which` (AMG_MATRICES) of AMG level `level` -> scipy CSR in internal order, values as double."""
+        import scipy.sparse as sp
+        k = C.c_int(self.AMG_MATRICES[which])
+        nnz = C.c_int64(0)
+        _check(self.lib.shakti_amg_get_matrix(self._h, C.c_int(level), k, None, None, None, C.byref(nnz)))
+        info = self.amg_level_info(level)
+        rows, cols = info["rows"], info["cols"]
+        if which == "P":
+            cols = info["n_coarse"]
+        elif which == "R":
+            rows = info["n_coarse"]
+        rowptr = np.empty(rows + 1, dtype=np.int32)
+        col = np.empty(nnz.value, dtype=np.int32)
+        val = np.empty(nnz.value)
+        _check(self.lib.shakti_amg_get_matrix(self._h, C.c_int(level), k, _p(rowptr), _p(col), _p(val), C.byref(nnz)))
+        return sp.csr_matrix((val, col, rowptr), shape=(rows, cols))
+
+    def amg_vectors(self, level):
+        """-> dict(dinv, dinv_cycle, lmax, coef) of AMG level `level` (coef: empty without the Chebyshev smoother)."""
+        n = self.amg_level_info(level)["rows"]
+        dinv, dc = np.empty(n), np.empty(n)
+        lmax, stride = C.c_double(0), C.c_int32(0)
+        _check(self.lib.shakti_amg_get_vectors(self._h, C.c_int(level), None, None, None, None, C.byref(stride)))
+        coef = np.empty(stride.value)
+        _check(self.lib.shakti_amg_get_vectors(self._h, C.c_int(level), _p(dinv), _p(dc), C.byref(lmax), _p(coef),
+                                               C.byref(stride)))
+        return dict(dinv=dinv, dinv_cycle=dc, lmax=lmax.value, coef=coef)
+
+    def amg_apply(self, r):
+        """z = M^-1 r: one V-cycle on owned-length vectors in internal order, as a Krylov iteration applies it."""
+        r = _f64(r)
+        z = np.empty_like(r)
+        _check(self.lib.shakti_amg_apply(self._h, _p(r), _p(z)))
+        return z
