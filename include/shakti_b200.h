@@ -272,19 +272,21 @@ int shakti_free_pinned(void* p);
  * use the assembly's own quadrature; every value is global (summed / reduced over ranks).  With F~ the residual
  * without Dirichlet replacement or lifting, sum_i F~_i = int R, which splits into the identity
  *   outflow = input - (1/rho_i - 1/rho_w) melt + closure + storage + imbalance
- * that holds at every converged step up to rounding (DESIGN.md, "Water-budget diagnostics"). */
+ * that holds at every converged step up to rounding (DESIGN.md, "Water-budget diagnostics").  With moulins,
+ * sum_i F~_i = int R - sum_k Q_k(t), so the moulin discharge at the solve's time t = model time + dt is part of
+ * `input` (each rank adds its own moulins). */
 typedef enum shakti_diag {
   SHAKTI_D_DT = 0,          /* dt of the solve [s]                                          */
   SHAKTI_D_NEWTON_ITS = 1,  /* Newton iterations                                            */
   SHAKTI_D_RESIDUAL = 2,    /* ||F||_2 at exit (stats.last_residual)                        */
   SHAKTI_D_AREA = 3,        /* int 1 [m^2]                                                  */
   SHAKTI_D_WATER_VOLUME = 4,/* int b [m^3]                                                  */
-  SHAKTI_D_INPUT = 5,       /* int inputs [m^3/s]                                           */
+  SHAKTI_D_INPUT = 5,       /* int inputs + sum_k Q_k(t) of the moulins [m^3/s] (no moulins: int inputs) */
   SHAKTI_D_MELT = 6,        /* int (m0 + mdiff) [kg/s]                                      */
   SHAKTI_D_CLOSURE = 7,     /* int A b N|N|^(n-1) [m^3/s]                                   */
   SHAKTI_D_STORAGE = 8,     /* int storage (N - N_n) / (rho_w g dt) [m^3/s]                 */
   SHAKTI_D_OUTFLOW = 9,     /* -sum over Dirichlet rows of F~: discharge through the boundary [m^3/s] */
-  SHAKTI_D_IMBALANCE = 10,  /* sum over the other rows of F~: what Newton left [m^3/s]      */
+  SHAKTI_D_IMBALANCE = 10,  /* sum over the other rows of F~ (moulin rows included): what Newton left [m^3/s] */
   SHAKTI_D_N_MEAN = 11,     /* int N / int 1 [Pa]                                           */
   SHAKTI_D_N_MIN = 12,      /* min over vertices [Pa]                                       */
   SHAKTI_D_N_MAX = 13,      /* max over vertices [Pa]                                       */
@@ -303,6 +305,31 @@ int shakti_record_diagnostics(shakti_model* m, int64_t capacity);
 /* Copy the recorded rows (row-major, SHAKTI_D_COUNT doubles each; max_rows must hold them all) to `rows` and
  * empty the buffer; *n_rows = rows copied.  rows == NULL: only query the count (the buffer is kept). */
 int shakti_read_diagnostics(shakti_model* m, double* rows, int64_t max_rows, int64_t* n_rows);
+
+/* ---------------------------------------------------------------- moulins (point water inputs)
+ * Extension: the reference's only water input is the distributed field md.inputs (solvers.py:45).  A moulin is a
+ * caller vertex v_k with a piecewise-linear hydrograph Q_k(t) [m^3/s]: knots (t_j, Q_j) with t_j strictly
+ * increasing, linear between knots, constant outside them.  period > 0 first wraps t into [t_0, t_0 + period) of
+ * each hydrograph (diurnal cycles); 0 means no period.  After every assembly
+ *   F_i -= sum over k with v_k = i of Q_k(t)       (moulins of one vertex summed in the order given, no atomics)
+ * -- the source term of solvers.py:45 with a Dirac right-hand side, the sign of the `- inputs` term.  The Jacobian
+ * is unchanged.  The model keeps a clock: a Newton solve (and shakti_assemble / shakti_diagnostics) with step dt
+ * evaluates Q at model time + dt, the end of the step; shakti_update_b (which closes a step) advances the clock
+ * by dt; shakti_snapshot / shakti_rollback save and restore it.  It starts at 0.
+ * A moulin may not sit on a Dirichlet dof: shakti_set_moulins refuses one, and so does a later
+ * shakti_set_dirichlet that would create one.  On several GPUs every rank passes the same (global) list; each rank
+ * applies the moulins of the vertices it owns.  Without moulins a step launches exactly what it did before. */
+/* n_moulins moulins: vertex[k] (caller id); the knots of moulin k are t_knots / q_knots [knot_ptr[k],
+ * knot_ptr[k+1]), knot_ptr[0] = 0 (n_moulins + 1 entries).  Replaces the previous set; n_moulins = 0 removes all.
+ * Invalid arguments (vertex out of range or on a Dirichlet dof, an empty hydrograph, non-increasing knot times,
+ * NaN or Inf, a negative period) return SHAKTI_ERR_INVALID and leave the model unchanged. */
+int shakti_set_moulins(shakti_model* m, int64_t n_moulins, const int32_t* vertex, const int64_t* knot_ptr,
+                       const double* t_knots, const double* q_knots, double period);
+/* The model clock [s] (finite). */
+int shakti_set_time(shakti_model* m, double t);
+int shakti_get_time(shakti_model* m, double* t);
+/* Parity hook: q_out[k] = Q_k(t) in caller order, evaluated on the host with the device's arithmetic. */
+int shakti_moulin_discharge(shakti_model* m, double t, double* q_out);
 
 /* Diagnostic: GB/s of cudaMemcpyAsync host->device / device->host for `host` (any host pointer) and the host
  * milliseconds each enqueue took (enqueue_ms[0] h2d, [1] d2h): tells page-locked from pageable memory. */

@@ -69,6 +69,21 @@ struct shakti_model {
   DevBuf<double> diag_partial, diag_vals, diag_rows;
   int diag_parts = 1;
   int64_t diag_cap = 0, diag_n = 0, snap_diag_n = 0;
+  // model clock [s]: a solve with step dt is forced at t_model + dt; update_b advances it by dt
+  double t_model = 0.0, snap_t_model = 0.0;
+  // moulins (shakti_set_moulins): every moulin in caller order on the host (mo_kptr/mo_t/mo_q: CSR of the knots),
+  // this rank's moulins on the device grouped by row (MoulinView), mo_own: their caller indices in that order
+  int64_t n_moulins = 0;
+  std::vector<int32_t> mo_vertex;
+  std::vector<int64_t> mo_kptr;
+  std::vector<double> mo_t, mo_q;
+  double mo_period = 0.0;
+  std::vector<int64_t> mo_own;
+  int32_t mo_rows = 0;
+  DevBuf<int32_t> mo_row_d, mo_rptr_d;
+  DevBuf<int64_t> mo_kptr_d;
+  DevBuf<double> mo_t_d, mo_q_d;
+  std::vector<int32_t> bc_g;   // Dirichlet dofs (caller ids, sorted)
   double N_bdry = 0.0;
   int64_t n_bc = 0;
   bool h0_dirty = true;
@@ -194,6 +209,26 @@ static void compute_kbar(shakti_model* m) {
               m->dprm, m->stream);
 }
 
+static MoulinView moulin_view(const shakti_model* m) {
+  return {m->mo_rows, m->mo_row_d.p, m->mo_rptr_d.p, m->mo_kptr_d.p, m->mo_t_d.p, m->mo_q_d.p, m->mo_period};
+}
+
+// F -= moulin discharge at the end of the step (t_model + dt).  Moulin rows are never Dirichlet rows, so this
+// commutes with the Dirichlet replacement, and the Jacobian is unchanged.
+static void apply_moulins(shakti_model* m, double dt) {
+  if (m->n_moulins > 0) launch_moulin_source(moulin_view(m), m->t_model + dt, m->F.p, m->stream);
+}
+
+// total discharge of this rank's moulins at t, on the host (the same bits as the device evaluation)
+static double owned_moulin_discharge(const shakti_model* m, double t) {
+  double s = 0.0;
+  for (int64_t k : m->mo_own) {
+    const int64_t a = m->mo_kptr[k];
+    s += hydrograph_at(m->mo_t.data() + a, m->mo_q.data() + a, m->mo_kptr[k + 1] - a, m->mo_period, t);
+  }
+  return s;
+}
+
 // residual (+ Jacobian) at the current state; Kbar must be current
 static void assemble(shakti_model* m, double dt, int want_J) {
   SHAKTI_PHASE(want_J ? "assembleFJ" : "assembleF", m->stream);
@@ -205,6 +240,7 @@ static void assemble(shakti_model* m, double dt, int want_J) {
                         m->ab_elems.p, m->ab_lv.p, m->ab_hptr.p, m->ab_halo.p, m->ab_incptr.p, m->ab_inc.p, m->ab_src.p};
     launch_assemble_blocks(pl, m->fields(), m->kbar.p, dt, m->N_bdry, m->J.slice_ptr.p, m->F.p, m->J.val.p, want_J, m->dprm,
                            m->stream);
+    apply_moulins(m, dt);
     if (want_J) m->J_valid = true;
     return;
   }
@@ -213,6 +249,7 @@ static void assemble(shakti_model* m, double dt, int want_J) {
   launch_assemble_atomic(m->hm.ne, no, m->c0.p, m->c1.p, m->c2.p, m->slot.p, m->fields(), m->kbar.p, dt,
                          m->N_bdry, m->F.p, m->J.val.p, want_J, m->dprm, m->stream);
   if (m->n_bc) launch_apply_bc(no, m->isbc.p, m->N.p, m->N_bdry, m->diag_pos.p, m->F.p, m->J.val.p, want_J, m->stream);
+  apply_moulins(m, dt);
   if (want_J) m->J_valid = true;
 }
 
@@ -337,17 +374,20 @@ __global__ void fix_bc_dx_kernel(int32_t n, const uint8_t* __restrict__ isbc, co
 // are those of the exact iteration (tests: identical Newton counts, fields <= 1e-8 against the CPU LU
 // restatement) at roughly 60 % of the Krylov iterations.
 // One water-budget record of the current state into `row` (device, SHAKTI_D_COUNT doubles), on the stream.
-// Kbar and h0 must be current.
+// Kbar and h0 must be current.  With moulins, each rank adds the discharge of its own moulins at t_model + dt
+// (the time the residual is forced at) before the reduction.
 static void diagnostics_record(shakti_model* m, double dt, int its, double residual, double* row) {
   ensure_rules(m);
-  const bool multi = comm().active();
+  const bool multi = comm().active(), moulins = m->n_moulins > 0;
   launch_diagnostics(m->hm.ne, m->c0.p, m->c1.p, m->c2.p, m->cell_counted.p, m->fields(), m->kbar.p, dt, m->dprm,
-                     m->diag_parts, m->diag_partial.p, m->diag_vals.p, multi ? nullptr : row, its, residual, m->stream);
+                     m->diag_parts, m->diag_partial.p, m->diag_vals.p, multi || moulins ? nullptr : row, its, residual,
+                     m->stream);
+  if (moulins) launch_diagnostics_moulins(m->diag_vals.p, owned_moulin_discharge(m, m->t_model + dt), m->stream);
   if (multi) {
     comm_allreduce_sum(m->diag_vals.p, kDiagSums, m->stream);
     comm_allreduce_max(m->diag_vals.p + kDiagSums, kDiagVals - kDiagSums, m->stream);
-    launch_diagnostics_row(m->diag_vals.p, row, dt, its, residual, m->stream);
   }
+  if (multi || moulins) launch_diagnostics_row(m->diag_vals.p, row, dt, its, residual, m->stream);
 }
 
 static void require_diag_rows(shakti_model* m, int64_t n) {
@@ -500,8 +540,10 @@ static void update_b(shakti_model* m, double dt) {
   m->halo.exchange(m->qx.p, m->stream);
   m->halo.exchange(m->qy.p, m->stream);
   // the gap-height update closes a time step on both paths (shakti_step and the split entry points
-  // solvers.solve(md) drives), so the step counter -- and with it amg_refresh_every -- advances here
+  // solvers.solve(md) drives), so the step counter -- and with it amg_refresh_every -- advances here, and so does
+  // the model clock
   m->st.steps++;
+  m->t_model += dt;
 }
 static void copy_N(shakti_model* m) {
   SHAKTI_CUDA(cudaMemcpyAsync(m->N_n.p, m->N.p, sizeof(double) * m->hm.n_local, cudaMemcpyDeviceToDevice, m->stream));
@@ -559,6 +601,8 @@ static void save_outputs_async(shakti_model* m, double* b_out, double* N_out, do
   m->d2h_pending = true;
 }
 
+static bool is_dirichlet(const shakti_model* m, int32_t v) { return std::binary_search(m->bc_g.begin(), m->bc_g.end(), v); }
+
 static void set_dirichlet(shakti_model* m, const int32_t* dofs, int64_t n, double value) {
   std::vector<uint8_t> flag(m->hm.n_local, 0);
   for (int64_t i = 0; i < n; ++i) {
@@ -566,12 +610,73 @@ static void set_dirichlet(shakti_model* m, const int32_t* dofs, int64_t n, doubl
     const int32_t l = m->hm.g2l[dofs[i]];
     if (l >= 0) flag[l] = 1;
   }
+  std::vector<int32_t> bc(dofs, dofs + n);
+  std::sort(bc.begin(), bc.end());
+  for (int64_t k = 0; k < m->n_moulins; ++k)
+    if (std::binary_search(bc.begin(), bc.end(), m->mo_vertex[k]))
+      throw Error(SHAKTI_ERR_INVALID, "Dirichlet dof " + std::to_string(m->mo_vertex[k]) + " carries moulin " +
+                                          std::to_string(k) + ": remove or move the moulin first");
+  m->bc_g.swap(bc);
   m->isbc.upload(flag);
   m->N_bdry = value;
   m->n_bc = n;   // global count: >0 on every rank
   m->hist_ratio = -1.0;
   m->amg_setup_done = false;  // excluded rows changed
   m->amg.reset();
+}
+
+// Validate everything before any state changes; then keep the hydrographs on the host and upload this rank's
+// moulin rows (owned vertices only: ghosts belong to another rank) sorted by row, caller order within a row.
+static void set_moulins(shakti_model* m, int64_t n, const int32_t* vertex, const int64_t* knot_ptr, const double* t_knots,
+                        const double* q_knots, double period) {
+  SHAKTI_REQUIRE(n >= 0 && n < ((int64_t)1 << 31), "n_moulins out of range");
+  SHAKTI_REQUIRE(std::isfinite(period) && period >= 0, "moulin period must be finite and >= 0 (0: no period)");
+  if (n > 0) SHAKTI_REQUIRE(vertex && knot_ptr && t_knots && q_knots, "null moulin argument");
+  if (n > 0) SHAKTI_REQUIRE(knot_ptr[0] == 0, "knot_ptr[0] must be 0");
+  for (int64_t k = 0; k < n; ++k) {
+    const std::string who = "moulin " + std::to_string(k);
+    SHAKTI_REQUIRE(vertex[k] >= 0 && vertex[k] < m->hm.nv_g, who + ": vertex out of range");
+    if (is_dirichlet(m, vertex[k]))
+      throw Error(SHAKTI_ERR_INVALID, who + ": vertex " + std::to_string(vertex[k]) + " is a Dirichlet dof");
+    SHAKTI_REQUIRE(knot_ptr[k + 1] > knot_ptr[k], who + ": empty hydrograph");
+    for (int64_t j = knot_ptr[k]; j < knot_ptr[k + 1]; ++j) {
+      SHAKTI_REQUIRE(std::isfinite(t_knots[j]) && std::isfinite(q_knots[j]), who + ": knot times and discharges must be finite");
+      SHAKTI_REQUIRE(j == knot_ptr[k] || t_knots[j] > t_knots[j - 1], who + ": knot times must be strictly increasing");
+    }
+  }
+  const int64_t nk = n > 0 ? knot_ptr[n] : 0;
+  std::vector<int64_t> own;
+  for (int64_t k = 0; k < n; ++k) {
+    const int32_t l = m->hm.g2l[vertex[k]];
+    if (l >= 0 && l < m->hm.n_owned) own.push_back(k);
+  }
+  std::stable_sort(own.begin(), own.end(), [&](int64_t a, int64_t b) { return m->hm.g2l[vertex[a]] < m->hm.g2l[vertex[b]]; });
+  std::vector<int32_t> row, rptr;
+  std::vector<int64_t> kptr(1, 0);
+  std::vector<double> tk, qk;
+  for (size_t i = 0; i < own.size(); ++i) {
+    const int64_t k = own[i];
+    const int32_t l = m->hm.g2l[vertex[k]];
+    if (row.empty() || row.back() != l) { row.push_back(l); rptr.push_back((int32_t)i); }
+    tk.insert(tk.end(), t_knots + knot_ptr[k], t_knots + knot_ptr[k + 1]);
+    qk.insert(qk.end(), q_knots + knot_ptr[k], q_knots + knot_ptr[k + 1]);
+    kptr.push_back((int64_t)tk.size());
+  }
+  rptr.push_back((int32_t)own.size());
+  SHAKTI_CUDA(cudaStreamSynchronize(m->stream));   // a queued assembly may still read the old tables
+  m->mo_row_d.upload(row);
+  m->mo_rptr_d.upload(rptr);
+  m->mo_kptr_d.upload(kptr);
+  m->mo_t_d.upload(tk);
+  m->mo_q_d.upload(qk);
+  m->mo_rows = (int32_t)row.size();
+  m->n_moulins = n;
+  m->mo_vertex.assign(vertex, vertex + n);
+  m->mo_kptr.assign(knot_ptr, knot_ptr + n + (n > 0));
+  m->mo_t.assign(t_knots, t_knots + nk);
+  m->mo_q.assign(q_knots, q_knots + nk);
+  m->mo_period = period;
+  m->mo_own.swap(own);
 }
 
 static HostCsr& caller_pattern(shakti_model* m) {
@@ -1170,6 +1275,7 @@ int shakti_snapshot(shakti_model* m) {
   }
   m->snap_hist_ratio = m->hist_ratio; m->snap_hist_dt = m->hist_dt; m->snap_residual0 = m->residual0;
   m->snap_steps = m->st.steps;
+  m->snap_t_model = m->t_model;
   m->snap_diag_n = m->diag_n;
   m->snap_valid = true;
   SHAKTI_CATCH
@@ -1186,6 +1292,7 @@ int shakti_rollback(shakti_model* m) {
   m->hist_ratio = m->snap_hist_ratio; m->hist_dt = m->snap_hist_dt; m->residual0 = m->snap_residual0;
   // the step counter goes back too, and the AMG hierarchy (numbers of a later state) is renewed at the next solve
   m->st.steps = m->snap_steps;
+  m->t_model = m->snap_t_model;
   m->step_of_refresh = -1000000;
   m->diag_n = std::min(m->diag_n, m->snap_diag_n);   // records of the undone solves
   SHAKTI_CATCH
@@ -1229,6 +1336,39 @@ int shakti_read_diagnostics(shakti_model* m, double* rows, int64_t max_rows, int
                                 m->stream));
   SHAKTI_CUDA(cudaStreamSynchronize(m->stream));
   m->diag_n = m->snap_diag_n = 0;
+  SHAKTI_CATCH
+}
+
+int shakti_set_moulins(shakti_model* m, int64_t n_moulins, const int32_t* vertex, const int64_t* knot_ptr,
+                       const double* t_knots, const double* q_knots, double period) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m, "null model");
+  use_device(m);
+  shakti::set_moulins(m, n_moulins, vertex, knot_ptr, t_knots, q_knots, period);
+  SHAKTI_CATCH
+}
+
+int shakti_set_time(shakti_model* m, double t) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && std::isfinite(t), "bad arguments: the model time must be finite");
+  m->t_model = t;
+  SHAKTI_CATCH
+}
+
+int shakti_get_time(shakti_model* m, double* t) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && t, "null argument");
+  *t = m->t_model;
+  SHAKTI_CATCH
+}
+
+int shakti_moulin_discharge(shakti_model* m, double t, double* q_out) {
+  SHAKTI_TRY
+  SHAKTI_REQUIRE(m && std::isfinite(t) && (q_out || m->n_moulins == 0), "bad arguments");
+  for (int64_t k = 0; k < m->n_moulins; ++k) {
+    const int64_t a = m->mo_kptr[k];
+    q_out[k] = hydrograph_at(m->mo_t.data() + a, m->mo_q.data() + a, m->mo_kptr[k + 1] - a, m->mo_period, t);
+  }
   SHAKTI_CATCH
 }
 

@@ -3,6 +3,7 @@
 #include <cuda_fp16.h>
 
 #include "common.h"
+#include "moulin.h"
 #include "prep.h"
 #include "sell_row.h"
 
@@ -99,6 +100,20 @@ void launch_diagnostics(int32_t ne, const int32_t* c0, const int32_t* c1, const 
                         double its, double residual, cudaStream_t s);
 // record row from globally reduced vals (several ranks)
 void launch_diagnostics_row(const double* vals, double* row, double dt, double its, double residual, cudaStream_t s);
+// rank values: input += q, imbalance -= q (q: discharge of this rank's moulins)
+void launch_diagnostics_moulins(double* vals, double q, cudaStream_t s);
+
+// ---- moulins (shakti_set_moulins): this rank's moulin rows, each with its moulins in caller order
+struct MoulinView {
+  int32_t n_rows;
+  const int32_t* row;    // n_rows local row ids (owned), ascending
+  const int32_t* rptr;   // n_rows + 1: moulins of row r are rptr[r] .. rptr[r+1]-1
+  const int64_t* kptr;   // moulins + 1: knots of moulin k are kptr[k] .. kptr[k+1]-1 of tk, qk
+  const double *tk, *qk;
+  double period;
+};
+// F[row] -= sum over the row's moulins of Q_k(t)   (moulin.h hydrograph_at)
+void launch_moulin_source(const MoulinView& mv, double t, double* F, cudaStream_t s);
 
 // ---- nodal updates (solvers.py:186-197)
 void launch_update_q(int32_t n_owned, const int32_t* win, const double* x, const double* y,

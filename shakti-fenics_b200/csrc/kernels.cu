@@ -1453,4 +1453,36 @@ void launch_diagnostics_row(const double* vals, double* row, double dt, double i
   SHAKTI_LAUNCH(diagnostics_row_kernel, 1, 1, 0, s, vals, row, dt, its, residual);
 }
 
+// the moulin discharge q enters the input and, through F, the imbalance (DESIGN.md "Moulins")
+__global__ void diagnostics_moulin_kernel(double* __restrict__ vals, double q) {
+  vals[kDiagInput] += q;
+  vals[kDiagImbalance] -= q;
+}
+
+void launch_diagnostics_moulins(double* vals, double q, cudaStream_t s) {
+  SHAKTI_LAUNCH(diagnostics_moulin_kernel, 1, 1, 0, s, vals, q);
+}
+
+// ------------------------------------------------------------------ moulins
+// F[row[r]] -= sum of the hydrographs of moulins rptr[r] .. rptr[r+1]-1 at t, summed in that (caller) order: one
+// thread per row and no atomics, so F is bitwise reproducible.
+__global__ void moulin_source_kernel(int32_t n_rows, const int32_t* __restrict__ row, const int32_t* __restrict__ rptr,
+                                     const int64_t* __restrict__ kptr, const double* __restrict__ tk,
+                                     const double* __restrict__ qk, double period, double t, double* __restrict__ F) {
+  const int32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_rows) return;
+  double q = 0.0;
+  for (int32_t k = rptr[r]; k < rptr[r + 1]; ++k) {
+    const int64_t a = kptr[k];
+    q += hydrograph_at(tk + a, qk + a, kptr[k + 1] - a, period, t);
+  }
+  F[row[r]] -= q;
+}
+
+void launch_moulin_source(const MoulinView& mv, double t, double* F, cudaStream_t s) {
+  if (mv.n_rows == 0) return;
+  SHAKTI_LAUNCH(moulin_source_kernel, div_up(mv.n_rows, 128), 128, 0, s, mv.n_rows, mv.row, mv.rptr, mv.kptr, mv.tk, mv.qk,
+                mv.period, t, F);
+}
+
 }  // namespace shakti

@@ -498,6 +498,46 @@ class Model:
         _check(self.lib.shakti_read_diagnostics(self._h, _p(rows), C.c_int64(n.value), C.byref(n)))
         return rows[: n.value]
 
+    # ---- moulins (point water inputs with hydrographs; see shakti_set_moulins in the header)
+    def set_moulins(self, vertex, times, discharges, period=0.0, knot_ptr=None):
+        """Moulin k at caller vertex ``vertex[k]`` with hydrograph knots ``(times[k][j], discharges[k][j])`` [s, m^3/s].
+        ``times`` / ``discharges`` are ragged lists (one sequence per moulin), or flat arrays with ``knot_ptr`` (CSR,
+        len(vertex) + 1 entries).  ``period`` > 0 wraps t into [t_0, t_0 + period) of each hydrograph.  An empty
+        ``vertex`` removes every moulin."""
+        v = _i32(vertex).reshape(-1)
+        if knot_ptr is None:
+            if len(times) != v.size or len(discharges) != v.size:
+                raise ValueError("one hydrograph (times, discharges) per moulin")
+            lens = [np.size(t) for t in times]
+            if any(np.size(q) != n for q, n in zip(discharges, lens)):
+                raise ValueError("times and discharges of a moulin differ in length")
+            kp = np.zeros(v.size + 1, dtype=np.int64)
+            kp[1:] = np.cumsum(lens)
+            tk = _f64(np.concatenate([np.ravel(t) for t in times]) if v.size else np.zeros(0))
+            qk = _f64(np.concatenate([np.ravel(q) for q in discharges]) if v.size else np.zeros(0))
+        else:
+            kp = np.ascontiguousarray(knot_ptr, dtype=np.int64)
+            tk, qk = _f64(times).reshape(-1), _f64(discharges).reshape(-1)
+            if kp.size != v.size + 1 or tk.size != qk.size or (v.size and (kp[0] != 0 or kp[-1] != tk.size)):
+                raise ValueError("knot_ptr must have len(vertex) + 1 entries from 0 to the number of knots")
+        _check(self.lib.shakti_set_moulins(self._h, C.c_int64(v.size), _p(v), _p(kp), _p(tk), _p(qk), C.c_double(period)))
+        self.n_moulins = int(v.size)
+
+    def set_time(self, t):
+        """Model clock [s]: a solve with step dt is forced at t + dt; update_b advances the clock by dt."""
+        _check(self.lib.shakti_set_time(self._h, C.c_double(t)))
+
+    def get_time(self):
+        t = C.c_double(0)
+        _check(self.lib.shakti_get_time(self._h, C.byref(t)))
+        return t.value
+
+    def moulin_discharge(self, t):
+        """Q_k(t) of every moulin, in the order given to set_moulins."""
+        q = np.empty(getattr(self, "n_moulins", 0))
+        _check(self.lib.shakti_moulin_discharge(self._h, C.c_double(t), _p(q)))
+        return q
+
     # ---- micro-benchmarks
     KERNELS = dict(spmv=0, assemble=1, kbar=2, nodal=3, dot=4, axpy=5)
 

@@ -150,6 +150,41 @@ def cooke2_like(nsteps=87600, seed=2024):
     return c
 
 
+DAY = 86400.0
+
+
+def diurnal_hydrograph(q_mean, r, knots_per_day=24):
+    """Periodic table (times, Q) of max(0, q_mean (1 - r sin 2 pi t / day)) over one day, both ends included."""
+    t = np.linspace(0.0, DAY, knots_per_day + 1)
+    return t, np.maximum(0.0, q_mean * (1.0 - r * np.sin(2 * np.pi * t / DAY)))
+
+
+def moulins_like(nx=100, ny=20, n_moulins=60, nsteps=48, seed=7, r=1.2, q_total=60.0):
+    """SHMIP-like moulin run (the SHMIP moulin position files are not shipped, so this is seeded, not SHMIP):
+    100 km x 20 km ice-sheet margin with the SHMIP square-root surface and a flat bed, outflow at x = 0, a small
+    background input and `n_moulins` moulins at seeded positions in 10-90 km.  Each moulin gets a diurnal
+    hydrograph max(0, Qbar_k (1 - r sin 2 pi t / day)) tabulated hourly with period one day; the mean discharges
+    Qbar_k are seeded and sum to about q_total [m^3/s].  One-hour steps.  meta["moulins"]: (x, y, times, Q) tuples,
+    meta["moulin_period"]: the period."""
+    lx, ly = 100e3, 20e3
+    rng = np.random.default_rng(seed)
+    xy, cells = meshgen.rectangle(nx, ny, lx, ly, jitter=0.2, seed=seed, diagonal="alternate")
+    nv = xy.shape[0]
+    x = xy[:, 0]
+    z_s = 6.0 * (np.sqrt(x + 5e3) - np.sqrt(5e3)) + 1.0
+    f = dict(z_b=np.zeros(nv), z_s=z_s, G=np.full(nv, 0.05), inputs=np.full(nv, 7.93e-11), storage=np.zeros(nv),
+             b=np.full(nv, 0.05), N_n=np.full(nv, 1e5), q=np.zeros((nv, 2)), melt_n=np.zeros(nv))
+    mx = rng.uniform(0.1 * lx, 0.9 * lx, size=n_moulins)
+    my = rng.uniform(0.05 * ly, 0.95 * ly, size=n_moulins)
+    qbar = rng.uniform(0.5, 1.5, size=n_moulins)
+    qbar *= q_total / qbar.sum()
+    moulins = [(float(a), float(b), *diurnal_hydrograph(q, r)) for a, b, q in zip(mx, my, qbar)]
+    t = np.linspace(0.0, 3600.0 * (nsteps - 1), nsteps)
+    n_bdry = 917 * 9.81 * z_s.min()            # water at atmospheric pressure under the 1 m thick front
+    return Case("moulins_like", xy, cells, f, _left_edge_dofs(nx, ny), n_bdry, t,
+                meta=dict(nx=nx, ny=ny, lx=lx, ly=ly, moulins=moulins, moulin_period=DAY))
+
+
 def apply_case(model, case):
     """Upload a Case into a capi.Model and perform solvers.py:48 (N <- N_n)."""
     for k in ("z_b", "z_s", "G", "inputs", "storage", "b", "N_n", "melt_n"):

@@ -74,6 +74,35 @@ def _ensure_device_comm(md):
     _comm_ready = True
 
 
+def moulin_forcing(md, bc_dofs):
+    """md.moulins -> (vertex ids, times, discharges) for capi.Model.set_moulins.  Each entry is (x, y, times, Q),
+    snapped to the nearest mesh vertex, or (vertex, times, Q).  A moulin on an outflow (Dirichlet) dof is an error:
+    the Dirichlet row would discard its water."""
+    from scipy.spatial import cKDTree
+    bc = set(np.asarray(bc_dofs).tolist())
+    tree = None
+    vertex, times, discharges = [], [], []
+    for k, entry in enumerate(md.moulins):
+        if len(entry) == 4:
+            x, y, t, q = entry
+            if tree is None:
+                tree = cKDTree(np.column_stack([md.x, md.y]))
+            v = int(tree.query([float(x), float(y)])[1])
+            where = f"at ({float(x):.6g}, {float(y):.6g}), snapped to vertex {v}"
+        elif len(entry) == 3:
+            v, t, q = entry
+            v = int(v)
+            where = f"at vertex {v}"
+        else:
+            raise ValueError(f"moulin {k}: expected (x, y, times, Q) or (vertex, times, Q), got {len(entry)} items")
+        if v in bc:
+            raise ValueError(f"moulin {k} {where} lies on the outflow boundary (a Dirichlet dof): move it inland")
+        vertex.append(v)
+        times.append(np.asarray(t, dtype=np.float64))
+        discharges.append(np.asarray(q, dtype=np.float64))
+    return np.asarray(vertex, dtype=np.int32), times, discharges
+
+
 class B200NewtonSolver:
     """What ``NewtonSolver(md.comm, NonlinearProblem(F, N, bcs))`` is in the reference
     (solvers.py:51-52): ``solve(N)`` runs the Newton iteration for the weak form of
@@ -101,8 +130,13 @@ class B200NewtonSolver:
                         ("b", b), ("N", N), ("N_n", N_n), ("melt_n", melt_n)):
             m.set_field(name, f.x.array)
         m.set_flux(q.x.array)
+        bc_dofs = np.concatenate([bc.dofs for bc in bcs]) if bcs else np.zeros(0, dtype=np.int32)
         if bcs:
-            m.set_dirichlet(np.concatenate([bc.dofs for bc in bcs]), bcs[0].value)
+            m.set_dirichlet(bc_dofs, bcs[0].value)
+        # extension (off unless the setup sets md.moulins): point water inputs with hydrographs, see moulin_forcing
+        if getattr(md, "moulins", None):
+            vertex, times, discharges = moulin_forcing(md, bc_dofs)
+            m.set_moulins(vertex, times, discharges, period=float(getattr(md, "moulin_period", 0.0)))
         self.sync_host = True       # copy N back into the Function after every solve
 
     def _push_newton_options(self):
@@ -368,6 +402,10 @@ def solve(md):
 
         if inputs_of_t is not None:
             solver.set_inputs(inputs_of_t(md.timesteps[i]))
+
+        # model clock: the solve below is forced at t + dt = md.timesteps[i], the time inputs_of_t uses.  It is set
+        # every step, so a resumed run needs nothing from the checkpoint for it.
+        solver.model.set_time(md.timesteps[i] - dt.value)
 
         # effective pressure
         niter, converged = solver.solve(N)
