@@ -11,6 +11,12 @@ def make_case(nx=24, ny=16, seed=0, scramble=True, storage=True, turbulent=True,
     xy, cells = meshgen.rectangle(nx, ny, 100e3, 50e3, jitter=0.25, seed=seed + 11, diagonal=diagonal)
     if scramble:
         xy, cells = meshgen.scramble(xy, cells, seed=seed + 5)
+    return case_on(xy, cells, seed, storage=storage, turbulent=turbulent, neg_b=neg_b)
+
+
+def case_on(xy, cells, seed=0, storage=True, turbulent=True, neg_b=False):
+    """The fields of make_case on any mesh of the 100 km x 50 km domain: storage on the disc of radius 15 km around
+    the centre, Dirichlet dofs on x = 0.  Returns (xy, cells, fields dict, bc_dofs, N_bdry)."""
     nv = xy.shape[0]
     x, y = xy[:, 0], xy[:, 1]
     rng = np.random.default_rng(seed)

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 import scipy.sparse as sp
 
+import unstructured
 from oracle.shakti_oracle import ShaktiOracle, csr_pattern, dirichlet_dofs
 from shakti_b200 import capi, meshgen
 
@@ -181,12 +182,17 @@ def test_product_never_imports_the_oracle():
             assert "oracle" not in f.read_text().lower(), f
 
 
-@pytest.mark.parametrize("nranks", [1, 2])
-def test_assembly_row_block_plan_emulated_in_numpy(mesh, nranks):
+# the rectangle, then the unstructured meshes of tests/unstructured.py (128-row blocks, 32-row blocks, refused)
+PLAN_MESHES = [("rectangle", 1), ("rectangle", 2)] + [(n, k) for n in ("U0", "U32", "UA") for k in (1, 2)]
+
+
+@pytest.mark.parametrize("name,nranks", PLAN_MESHES, ids=[str(k) if n == "rectangle" else f"{n}-{k}" for n, k in PLAN_MESHES])
+def test_assembly_row_block_plan_emulated_in_numpy(mesh, name, nranks):
     """The plan behind assemble_blocks_kernel (csrc/prep.cpp build_assembly_blocks), executed in numpy exactly
     as the kernel does -- stage the block's cells, then gather per row through the incident-cell codes and the
-    two-source codes -- must reproduce the plain scatter-add of the cell matrices, with no atomics."""
-    xy, cells = mesh
+    two-source codes -- must reproduce the plain scatter-add of the cell matrices, with no atomics.  On UA the
+    plan of the rank that owns the 500-triangle fan is refused (the atomic fallback runs there instead)."""
+    xy, cells = mesh if name == "rectangle" else unstructured.mesh(name)
     nv = xy.shape[0]
     o = ShaktiOracle(xy, cells)
     rng = np.random.default_rng(1)
@@ -197,10 +203,17 @@ def test_assembly_row_block_plan_emulated_in_numpy(mesh, nranks):
     Jref = sp.csr_matrix((ref, o.col, o.rowptr), shape=(nv, nv))
     Fref = np.zeros(nv)
     np.add.at(Fref, cells.ravel(), Fe.ravel())
+    refused = 0
     for r in range(nranks):
         hm = capi.HostMesh(xy, cells, r, nranks, 1)
         rb, nb, max_cells, max_verts, ok = hm.array("ab_info")
-        assert ok == 1 and rb in (32, 64, 128, 256) and max_cells <= 400
+        if nranks == 1 and name != "rectangle":
+            assert ((rb if ok else None), ok) == unstructured.PLAN[name, 1]
+        if not ok:
+            assert name == "UA"
+            refused += 1
+            continue
+        assert rb in (32, 64, 128, 256) and max_cells <= 400
         l2g, lc, cl2g = hm.array("l2g"), hm.array("cells").reshape(-1, 3), hm.array("cell_l2g")
         eptr, elems, lv = hm.array("ab_eptr"), hm.array("ab_elems"), hm.array("ab_lv").reshape(-1, 3)
         hptr, halo = hm.array("ab_hptr"), hm.array("ab_halo")
@@ -236,6 +249,7 @@ def test_assembly_row_block_plan_emulated_in_numpy(mesh, nranks):
         own = l2g[: hm.n_owned]
         assert np.allclose(F, Fref[own], rtol=1e-13, atol=1e-13)
         assert abs(_sell_to_csr(hm, vals, nv)[own] - Jref[own]).max() < 1e-12
+    assert refused == (1 if name == "UA" else 0)          # exactly the rank with the fan
 
 
 def test_symmetric_heap_allocator_selftest():
